@@ -2,6 +2,7 @@
 """bench.py -- throughput of the ft_grandprix hot path on B200 (contract: see DESIGN.md §Measurement).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload tick|lidar|step] [--cars C]
+    python bench.py ... --dump-outputs DIR      # also write the last timed step's arrays as DIR/<name>.npy
     python bench.py --impl reference ...        # the CPU arm (oracle port, all host threads)
 
 One "step" = one pass of the hot path over the whole fleet:
@@ -25,6 +26,7 @@ MuJoCo (`import mujoco`, also with baseline/_ref on sys.path).  If it imports, t
 restatement under oracle/ (kind "port").  The CPU arms never import the product package.
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -64,6 +66,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(self.index), f"--query-gpu={self.Q}",
                                           "--format=csv,noheader,nounits", "-lms", "100"],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)        # a run that fails before stop() must not leave nvidia-smi polling
             self.thread = threading.Thread(target=self._read, daemon=True)
             self.thread.start()
         except OSError:
@@ -111,6 +114,25 @@ def workload_name(wl, cars):
     return {"tick": f"full tick (lap + nidc + 90-beam lidar + vehicle step), {cars} cars/GPU on track.png (BASELINE config 3)",
             "lidar": f"lidar-only, {cars} cars/GPU at random poses on track.png, 90 beams, no cutoff (BASELINE config 2)",
             "step": f"vehicle step only, {cars} cars/GPU on track.png"}[wl]
+
+
+# what one call of the timed path hands back: the fleet arrays it writes
+TIMED_OUTPUTS = {"lidar": ("ranges",), "step": ("qpos", "qvel", "warm", "status")}
+TICK_OUTPUTS = ("qpos", "qvel", "warm", "ctrl", "ranges", "lap", "times", "winners", "status")
+DUMP_ROWS = 32768      # rows (cars, or worlds for `winners`) per array over all ranks: <= 45 MB of .npy files in all
+
+
+def dump_outputs(out_dir, fleet, wl, rank, world):
+    """--dump-outputs: the fleet arrays the timed path wrote in its last step, as out_dir/<name>.npy (float32 stays
+    float32, the integer arrays are widened to float64).  An array of more rows than its share of DUMP_ROWS is cut to a
+    fixed, seeded sample of rows, so that two builds run with the same arguments can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name in TIMED_OUTPUTS.get(wl, TICK_OUTPUTS):
+        a = getattr(fleet, name).cpu().numpy()
+        if len(a) > DUMP_ROWS // world:
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), DUMP_ROWS // world, replace=False))]
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
 
 
 # ----------------------------------------------------------------------------- CPU arms
@@ -183,8 +205,9 @@ def mujoco_units_per_s(mj, wl, ncars_model, ticks, seed=1):
 def cpu_units_per_s(wl, sample_cars, ticks, threads, seed=1):
     """Times the oracle (oracle/*.c, a C restatement: kind 'port') on a bounded sample of the workload."""
     from concurrent.futures import ThreadPoolExecutor
+    # the oracle library as build() left it: it is not re-made when oracle/*.c is newer (build() always runs make -B), and
+    # pyoracle.lib() makes it only if it is missing
     from oracle import pyoracle
-    pyoracle.build()
     wall, d_attr = bundled_track("track")
     ot = pyoracle.Track(wall)
     tpath = ot.centreline(d_attr)
@@ -322,6 +345,12 @@ def run_gpu(args):
             fleet.step(1)
             if kev: kev[3].record(stream)
 
+    def timed_step():
+        if wl == "tick":
+            fleet.tick(1)                # the product's fused entry point (ftgp_tick): same kernels, one C call
+        else:
+            one_step()
+
     stream = fleet.stream
     if wl == "tick" and args.fused_check:
         # the fused C entry point and the four separate calls are the same kernels in the same order
@@ -343,9 +372,9 @@ def run_gpu(args):
         settle = args.settle if wl != "lidar" else 0
         for k in range(settle):          # drive the fleet into its running regime (untimed)
             one_step()
-        for _ in range(args.warmup):
-            flush.fill_(1)
-            one_step()
+        for _ in range(args.warmup):     # warms the call that is timed: the first fused tick sets up its side stream and
+            flush.fill_(1)               # scratch, and small fleets capture their CUDA graph on the second one
+            timed_step()
     stream.synchronize()
 
     def barrier():
@@ -363,14 +392,13 @@ def run_gpu(args):
         for a, b in ev:
             flush.fill_(1)
             a.record(stream)
-            if wl == "tick":
-                fleet.tick(1)            # the product's fused entry point (ftgp_tick): same kernels, one C call
-            else:
-                one_step()
+            timed_step()
             b.record(stream)
     barrier()
     clocks = sampler.stop()
     launches = lib.ftgp_launch_count() - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, fleet, wl, rank, world)
     # second pass, same regime: the two heavy kernels bracketed by their own CUDA events on the launching stream
     with torch.cuda.stream(stream):
         for kev in kevs:
@@ -592,6 +620,8 @@ def run_episode(args, kind="episode"):
     barrier()
     clocks = sampler.stop()
     launches = lib.ftgp_launch_count() - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, fleet, kind, rank, world)
     dev_ms = e0.elapsed_time(e1)
     car_steps = float(n) * ticks_done
     t0 = time.perf_counter()
@@ -663,7 +693,9 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=50)
-    ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--warmup", type=int, default=5,
+                    help="untimed steps through the same call as the timed ones; fleets of up to 16,384 cars capture the tick's "
+                         "CUDA graph on its second call, so fewer than 2 leave that capture in the first timed step")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default=os.environ.get("FTGP_WORKLOAD", "tick"), choices=["tick", "lidar", "step", "episode", "race"])
     ap.add_argument("--cars", type=int, default=None)
@@ -673,7 +705,11 @@ def main():
     ap.add_argument("--lap-target", type=int, default=10)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--fused-check", action="store_true", help="assert that ftgp_tick == the four separate calls, bit for bit")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the arrays the timed path computed in its last step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; the reference arm has no such outputs")
     if args.cars is None:
         args.cars = {"lidar": 4096, "episode": 1048576, "race": 262144}.get(args.workload, 65536)
     if args.workload in ("episode", "race") and args.impl != "reference":

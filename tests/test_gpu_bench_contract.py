@@ -4,6 +4,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 from conftest import ROOT
@@ -42,6 +43,26 @@ def test_other_workloads_print_a_line(wl, cars):
     assert BASE <= set(d) and d["value"] > 0 and d["e2e"]["value"] > 0
     if wl in ("episode", "race"):
         assert d["scaling"] == "strong" and d["episode"]["stats_rows"] == int(cars)
+
+
+@pytest.mark.parametrize("cars", [40960, 4096])
+def test_dump_outputs_of_the_last_timed_tick(tmp_path, cars):
+    """--dump-outputs writes the fleet arrays of the last timed tick (40,960 cars: a seeded sample of 32,768 of them; 4,096
+    cars: all of them, the tick replayed as a CUDA graph), identical from run to run; 3 timed ticks after 5 settle ticks
+    end where 1 timed tick after 7 settle ticks ends."""
+    common = ("--cars", str(cars), "--warmup", "2", "--no-cpu-baseline", "--dump-outputs")
+    d = _run("--steps", "3", "--settle", "5", *common, str(tmp_path / "a"))
+    _run("--steps", "3", "--settle", "5", *common, str(tmp_path / "b"))
+    _run("--steps", "1", "--settle", "7", *common, str(tmp_path / "c"))
+    assert d["steps"] == 3
+    names = {"qpos", "qvel", "warm", "ctrl", "ranges", "lap", "times", "winners", "status"}
+    assert set(os.listdir(tmp_path / "a")) == {n + ".npy" for n in names}
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= 64 << 20
+    for n in names:
+        a, b, c = (np.load(tmp_path / r / (n + ".npy")) for r in "abc")
+        assert a.dtype == (np.float32 if n == "ranges" else np.float64) and len(a) == min(cars, 32768), n
+        assert np.array_equal(a, b) and np.array_equal(a, c), n
+    assert np.isfinite(np.load(tmp_path / "a" / "qpos.npy")).all()
 
 
 def test_reference_arm_line():
