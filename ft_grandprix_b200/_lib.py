@@ -13,6 +13,8 @@ NBEAMS, NQ, NV, NU, NPATH = 90, 34, 29, 2, 100
 MAX_TRACKS, MAX_LAPTIMES = 4, 16
 LAP_FIELDS = ("offset", "completion", "laps", "start", "good_start", "finished", "ntimes",
               "off_track", "rank", "delta", "offtrack_ticks", "contact_ticks")
+RACE_FIELDS = ("races", "finished", "wins", "rank_sum", "laps_sum", "time_sum", "best_lap", "offtrack_ticks",
+               "contact_ticks")
 DRIVER_NIDC, DRIVER_FAST, DRIVER_LOBOTOMY = 0, 1, 2
 OPT_NAIVE_FLATTEN, OPT_BUBBLE_WRAP = 1, 2
 
@@ -27,6 +29,10 @@ class TickArgs(C.Structure):
                 ("ncars", C.c_int64),
                 ("cars_per_world", C.c_int32), ("default_driver", C.c_int32),
                 ("lap_target", C.c_int32), ("steps", C.c_int32), ("options", C.c_int32), ("reserved", C.c_int32)]
+
+class ReloadArgs(C.Structure):
+    _fields_ = [("start_xy", C.c_void_p), ("start_yaw", C.c_void_p), ("start_offset", C.c_void_p),
+                ("race_start", C.c_void_p), ("tally", C.c_void_p), ("race_ticks", C.c_int32), ("reserved", C.c_int32)]
 
 _vp, _i, _i64, _d = C.c_void_p, C.c_int, C.c_int64, C.c_double
 # name -> (restype, argtypes); mirrors include/ftgp.h one to one
@@ -56,6 +62,8 @@ SIGNATURES = {
     "ftgp_tick": (_i, [C.POINTER(TickArgs), _i, _vp]),
     "ftgp_release_graphs": (_i, []),
     "ftgp_tick_use_graphs": (_i, [_i]),
+    "ftgp_reload": (_i, [C.POINTER(TickArgs), C.POINTER(ReloadArgs), _vp]),
+    "ftgp_tick_reload": (_i, [C.POINTER(TickArgs), C.POINTER(ReloadArgs), _i, _vp]),
 }
 
 _lib = None

@@ -6,6 +6,8 @@
 //                                                          ft_grandprix/lobotomy.py:1-3
 //                   + the control write                    ft_grandprix/custom.py:1418-1423
 //   lap_kernel      progress / lap state machine           ft_grandprix/custom.py:1340-1372
+//   reload_kernel   reload() of the worlds whose race is over, ft_grandprix/custom.py:1089-1128
+//                   with the race tally of their cars
 //
 // Layout: one warp per car for the driver (lane l owns beams l, l+32, l+64 of the 68-beam
 // front window, so the ranges row is read with coalesced 128-byte loads and the sequential
@@ -18,11 +20,8 @@
 namespace ftgp {
 
 // ------------------------------------------------------------------ reset
-__global__ void reset_kernel(double* __restrict__ qpos, double* __restrict__ qvel, double* __restrict__ warm,
-                             double* __restrict__ ctrl, const double* __restrict__ xy,
-                             const double* __restrict__ yaw, int64_t ncars) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= ncars) return;
+__device__ __forceinline__ void reset_car(int64_t i, double* __restrict__ qpos, double* __restrict__ qvel, double* __restrict__ warm,
+                                          double* __restrict__ ctrl, const double* __restrict__ xy, const double* __restrict__ yaw) {
     double* q = qpos + i * FTGP_NQ;
     // qpos0: free joint at the body pos (0, 2, 0) with identity quat, hinges/slides 0, balls identity
     // (mushr.em.xml:96); position_vehicles then overwrites x, y and the quaternion (custom.py:1244-1245)
@@ -34,6 +33,86 @@ __global__ void reset_kernel(double* __restrict__ qpos, double* __restrict__ qve
     q[11] = 1.0; q[18] = 1.0; q[24] = 1.0; q[30] = 1.0;          // ball joints of the four softener bodies
     for (int k = 0; k < FTGP_NV; k++) { qvel[i * FTGP_NV + k] = 0.0; warm[i * FTGP_NV + k] = 0.0; }
     if (ctrl) { ctrl[2 * i] = 0.0; ctrl[2 * i + 1] = 0.0; }
+}
+
+__global__ void reset_kernel(double* __restrict__ qpos, double* __restrict__ qvel, double* __restrict__ warm,
+                             double* __restrict__ ctrl, const double* __restrict__ xy,
+                             const double* __restrict__ yaw, int64_t ncars) {
+    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= ncars) return;
+    reset_car(i, qpos, qvel, warm, ctrl, xy, yaw);
+}
+
+// ------------------------------------------------------------------ reload of finished worlds (custom.py:1089-1128)
+// One thread per world, as the lap kernel: the due test reads the FINISHED flags of every car of the world and
+// race_start[w], and the reset writes both, so the thread that decides is the only one that writes the world (worlds of
+// 3, 5, 6 or 7 cars do not align to warps).  A world that is not due costs one int32 load (race_start, when race_ticks
+// decides) or the FINISHED flags up to the first car still racing, and no store.
+__global__ void reload_kernel(double* __restrict__ qpos, double* __restrict__ qvel, double* __restrict__ warm,
+                              double* __restrict__ ctrl, float* __restrict__ ranges, int32_t* __restrict__ lap,
+                              int32_t* __restrict__ times, int32_t* __restrict__ winners, int32_t* __restrict__ status,
+                              int64_t ncars, int cpw, const double* __restrict__ start_xy, const double* __restrict__ start_yaw,
+                              const int32_t* __restrict__ start_offset, int32_t* __restrict__ race_start,
+                              int32_t* __restrict__ tally, int32_t race_ticks, int32_t steps, const int32_t* __restrict__ steps_dev) {
+    const int64_t world = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t first = world * cpw;
+    if (first >= ncars) return;
+    const int64_t end = first + cpw < ncars ? first + cpw : ncars;
+    if (steps_dev) steps = *steps_dev;              // graph-replayed tick: the value the lap kernel reads after this one
+    bool due = race_ticks > 0 && (int64_t)steps - race_start[world] >= race_ticks;
+    if (!due) {
+        due = true;
+        for (int64_t car = first; car < end; car++)
+            if (!lap[car * FTGP_LAP_FIELDS + FTGP_LAP_FINISHED]) { due = false; break; }
+    }
+    if (!due) return;
+    for (int64_t car = first; car < end; car++) {
+        int32_t* s = lap + car * FTGP_LAP_FIELDS;
+        int32_t* tm = times + car * FTGP_MAX_LAPTIMES;
+        if (tally) {                                  // the race that just ended
+            int32_t* t = tally + car * FTGP_RACE_FIELDS;
+            const int nt = s[FTGP_LAP_NTIMES] < FTGP_MAX_LAPTIMES ? s[FTGP_LAP_NTIMES] : FTGP_MAX_LAPTIMES;
+            int32_t sum = 0, best = t[FTGP_RACE_BEST_LAP];
+            for (int k = 0; k < nt; k++) {
+                const int32_t v = tm[k];
+                sum += v;
+                if (v > 0 && (best == 0 || v < best)) best = v;
+            }
+            t[FTGP_RACE_RACES] += 1;
+            t[FTGP_RACE_FINISHED] += s[FTGP_LAP_FINISHED];
+            t[FTGP_RACE_WINS] += s[FTGP_LAP_RANK] == 1;
+            t[FTGP_RACE_RANK_SUM] += s[FTGP_LAP_RANK];
+            t[FTGP_RACE_LAPS_SUM] += s[FTGP_LAP_LAPS];
+            if (s[FTGP_LAP_FINISHED]) t[FTGP_RACE_TIME_SUM] += sum;
+            t[FTGP_RACE_BEST_LAP] = best;
+            t[FTGP_RACE_OFFTRACK_TICKS] += s[FTGP_LAP_OFFTRACK_TICKS];
+            t[FTGP_RACE_CONTACT_TICKS] += s[FTGP_LAP_CONTACT_TICKS];
+        }
+        // what Fleet.reset(xy, yaw) leaves: ftgp_reset, then ranges / lap / times / status zero, VehicleState(offset,
+        // good_start=True) (custom.py:96-118); START = steps keeps every lap time equal to a fresh fleet's
+        reset_car(car, qpos, qvel, warm, ctrl, start_xy, start_yaw);
+        for (int k = 0; k < FTGP_NBEAMS; k++) ranges[car * FTGP_NBEAMS + k] = 0.0f;
+        for (int k = 0; k < FTGP_MAX_LAPTIMES; k++) tm[k] = 0;
+        for (int k = 0; k < FTGP_LAP_FIELDS; k++) s[k] = 0;
+        s[FTGP_LAP_OFFSET] = start_offset[car];
+        s[FTGP_LAP_GOOD_START] = 1;
+        s[FTGP_LAP_START] = steps;
+        if (status) status[car] = 0;
+    }
+    if (winners) winners[world] = 0;
+    if (race_start) race_start[world] = steps;
+}
+
+int launch_reload(const ftgp_tick_args* a, const ftgp_reload_args* r, int32_t steps, cudaStream_t stream,
+                  const int32_t* steps_dev) {
+    const int64_t nworlds = (a->ncars + a->cars_per_world - 1) / a->cars_per_world;
+    const int threads = 128;
+    reload_kernel<<<(unsigned)((nworlds + threads - 1) / threads), threads, 0, stream>>>(
+        a->qpos, a->qvel, a->warm, a->ctrl, a->ranges, a->lap, a->times, a->winners, a->status, a->ncars, a->cars_per_world,
+        r->start_xy, r->start_yaw, r->start_offset, r->race_start, r->tally, r->race_ticks, steps, steps_dev);
+    count_launch();
+    FTGP_CUDA(cudaGetLastError());
+    return FTGP_OK;
 }
 
 // ------------------------------------------------------------------ option naive_flatten (custom.py:981,1338-1339)

@@ -464,6 +464,8 @@ int launch_lap(const ftgp_geom* g, const double* qpos, int64_t stride, const int
                int32_t lap_target, cudaStream_t stream, const int32_t* steps_dev);
 
 int launch_flatten(double* qpos, int64_t stride, int64_t ncars, cudaStream_t stream);
+int launch_reload(const ftgp_tick_args* a, const ftgp_reload_args* r, int32_t steps, cudaStream_t stream,
+                  const int32_t* steps_dev);
 
 // Inside the fused tick the rangefinder kernel runs on a side stream against a copy of the poses (mj_step
 // evaluates the rangefinders from the pre-step pose, custom.py:1425) while the vehicle step advances the state on the main
@@ -496,9 +498,11 @@ static int overlap_fork(double* qpos, int64_t ncars, bool copy, cudaStream_t str
     return FTGP_OK;
 }
 
-// ---- one tick = custom.py:1337-1426 for the whole fleet, in the reference's order
-static int issue_tick(const ftgp_tick_args* a, int32_t steps, int32_t* steps_dev, cudaStream_t s) {
+// ---- one tick = custom.py:1337-1426 for the whole fleet, in the reference's order; r != NULL: the worlds whose race is
+// over are reloaded first (custom.py:1089-1128)
+static int issue_tick(const ftgp_tick_args* a, const ftgp_reload_args* r, int32_t steps, int32_t* steps_dev, cudaStream_t s) {
     int rc;
+    if (r && (rc = launch_reload(a, r, steps, s, steps_dev))) return rc;
     // custom.py:1338-1339 option naive_flatten
     if ((a->options & FTGP_OPT_NAIVE_FLATTEN) && (rc = launch_flatten(a->qpos, FTGP_NQ, a->ncars, s))) return rc;
     // custom.py:1340-1372 progress + lap logic from the current pose
@@ -527,7 +531,7 @@ static int issue_tick(const ftgp_tick_args* a, int32_t steps, int32_t* steps_dev
 constexpr int64_t GRAPH_MAX_CARS = 16384;
 static std::atomic<int> g_use_graphs{1};
 struct TickGraph {
-    ftgp_tick_args key{}; cudaStream_t stream = nullptr; int dev = -1;
+    ftgp_tick_args key{}; bool reload = false; ftgp_reload_args rkey{}; cudaStream_t stream = nullptr; int dev = -1;
     cudaGraphExec_t exec = nullptr; int32_t* steps_dev = nullptr; int32_t shadow = INT32_MIN;
     uint64_t scratch_gen = 0; int launches_per_tick = 0; bool seen = false; uint64_t used = 0;
 };
@@ -547,6 +551,12 @@ static bool same_key(const ftgp_tick_args& x, const ftgp_tick_args& y) {
            x.winners == y.winners && x.status == y.status && x.ncars == y.ncars && x.cars_per_world == y.cars_per_world &&
            x.default_driver == y.default_driver && x.lap_target == y.lap_target && x.options == y.options;
 }
+static bool same_reload(const TickGraph& g, const ftgp_reload_args* r) {
+    if (!r) return !g.reload;
+    const ftgp_reload_args& x = g.rkey;
+    return g.reload && x.start_xy == r->start_xy && x.start_yaw == r->start_yaw && x.start_offset == r->start_offset &&
+           x.race_start == r->race_start && x.tally == r->tally && x.race_ticks == r->race_ticks;
+}
 static void drop_graph(TickGraph& g) {
     if (g.exec) cudaGraphExecDestroy(g.exec);
     if (g.steps_dev) cudaFree(g.steps_dev);
@@ -554,22 +564,24 @@ static void drop_graph(TickGraph& g) {
 }
 
 // returns FTGP_OK and sets *done = number of ticks issued through the graph (0: caller runs them eagerly)
-static int graph_ticks(const ftgp_tick_args* a, int nticks, cudaStream_t s, int* done) {
+static int graph_ticks(const ftgp_tick_args* a, const ftgp_reload_args* r, int nticks, cudaStream_t s, int* done) {
     *done = 0;
     int dev = 0;
     FTGP_CUDA(cudaGetDevice(&dev));
     std::lock_guard<std::mutex> lock(g_graph_mutex);
     TickGraph* e = nullptr; TickGraph* lru = &g_graphs[0];
     for (auto& g : g_graphs) {
-        if (g.seen && g.dev == dev && g.stream == s && same_key(g.key, *a)) { e = &g; break; }
+        if (g.seen && g.dev == dev && g.stream == s && same_key(g.key, *a) && same_reload(g, r)) { e = &g; break; }
         if (g.used < lru->used) lru = &g;
     }
     int32_t steps = a->steps;
     if (!e) {                                   // first tick with these arguments: register, run ONE tick eagerly
         drop_graph(*lru);
         lru->key = *a; lru->stream = s; lru->dev = dev; lru->seen = true;
+        lru->reload = r != nullptr;
+        if (r) lru->rkey = *r;
         e = lru;
-        const int rc = issue_tick(a, steps, nullptr, s);
+        const int rc = issue_tick(a, r, steps, nullptr, s);
         if (rc) return rc;
         steps++; nticks--; *done = 1;
         if (nticks == 0) { e->used = ++g_graph_clock; return FTGP_OK; }
@@ -582,7 +594,7 @@ static int graph_ticks(const ftgp_tick_args* a, int nticks, cudaStream_t s, int*
         const int64_t l0 = ftgp_launch_count();
         cudaGraph_t graph = nullptr;
         FTGP_CUDA(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-        const int rc = issue_tick(a, 0, e->steps_dev, s);
+        const int rc = issue_tick(a, r, 0, e->steps_dev, s);
         const cudaError_t ce = cudaStreamEndCapture(s, &graph);
         if (rc || ce != cudaSuccess || !graph) {                 // capture refused (e.g. scratch had to grow): stay eager
             if (graph) cudaGraphDestroy(graph);
@@ -627,19 +639,38 @@ extern "C" int ftgp_release_scratch(void* stream) {
     return FTGP_OK;
 }
 
-extern "C" int ftgp_tick(const ftgp_tick_args* a, int nticks, void* stream) {
-    if (!a || !a->geom || !a->qpos || !a->qvel || !a->warm || !a->ctrl || !a->ranges || !a->lap || !a->times ||
-        a->ncars < 0 || a->cars_per_world < 1 || nticks < 0) { set_error("ftgp_tick: bad argument"); return FTGP_ERR_ARG; }
+static bool bad_tick_args(const ftgp_tick_args* a) {
+    return !a || !a->geom || !a->qpos || !a->qvel || !a->warm || !a->ctrl || !a->ranges || !a->lap || !a->times ||
+           a->ncars < 0 || a->cars_per_world < 1;
+}
+// checked before any CUDA call: the race cap and the tally both need race_start
+static bool bad_reload_args(const ftgp_reload_args* r) {
+    return !r || !r->start_xy || !r->start_yaw || !r->start_offset || r->race_ticks < 0 ||
+           (r->tally && !r->race_start) || (r->race_ticks > 0 && !r->race_start);
+}
+
+extern "C" int ftgp_tick_reload(const ftgp_tick_args* a, const ftgp_reload_args* r, int nticks, void* stream) {
+    if (bad_tick_args(a) || nticks < 0) { set_error("ftgp_tick: bad argument"); return FTGP_ERR_ARG; }
+    if (r && bad_reload_args(r)) { set_error("ftgp_tick_reload: bad reload argument"); return FTGP_ERR_ARG; }
     if (a->ncars == 0 || nticks == 0) return FTGP_OK;
     FTGP_CUDA(cudaSetDevice(a->geom->device));
     cudaStream_t s = (cudaStream_t)stream;
     int t0 = 0, rc;
     if (a->ncars <= GRAPH_MAX_CARS && s != nullptr && g_use_graphs.load()) {           // (the legacy default stream cannot be captured)
-        if ((rc = graph_ticks(a, nticks, s, &t0))) return rc;
+        if ((rc = graph_ticks(a, r, nticks, s, &t0))) return rc;
     }
     for (int t = t0; t < nticks; t++)
-        if ((rc = issue_tick(a, a->steps + t, nullptr, s))) return rc;
+        if ((rc = issue_tick(a, r, a->steps + t, nullptr, s))) return rc;
     return FTGP_OK;
+}
+
+extern "C" int ftgp_tick(const ftgp_tick_args* a, int nticks, void* stream) { return ftgp_tick_reload(a, nullptr, nticks, stream); }
+
+extern "C" int ftgp_reload(const ftgp_tick_args* a, const ftgp_reload_args* r, void* stream) {
+    if (bad_tick_args(a) || bad_reload_args(r)) { set_error("ftgp_reload: bad argument"); return FTGP_ERR_ARG; }
+    if (a->ncars == 0) return FTGP_OK;
+    FTGP_CUDA(cudaSetDevice(a->geom->device));
+    return launch_reload(a, r, a->steps, (cudaStream_t)stream, nullptr);
 }
 
 extern "C" int ftgp_tick_use_graphs(int enable) { return g_use_graphs.exchange(enable ? 1 : 0); }

@@ -36,7 +36,7 @@ void count_launch(int n) { g_launches += n; }
 using namespace ftgp;
 
 extern "C" const char* ftgp_last_error(void) { return g_err; }
-extern "C" int ftgp_abi_version(void) { return 2; }
+extern "C" int ftgp_abi_version(void) { return 3; }
 extern "C" int64_t ftgp_launch_count(void) { return g_launches.load(); }
 
 extern "C" ftgp_track* ftgp_track_create(const uint8_t* px, int w, int h, int channels,

@@ -12,6 +12,8 @@ Mirrors what `Mujoco.physics_thread` touches every tick (ft_grandprix/custom.py:
     self.winners                                      fleet.lap[:, rank] / fleet.winners[world]
     mujoco.mj_step(model, data)                       fleet.step()
     driver.process_lidar(ranges)                      fleet.drive() (device) / fleet.drive_host()
+    reload() after every car has finished             Fleet(reload_finished=True): inside fleet.tick(), per world,
+                                                      race results summed in fleet.race_tally (RACE_FIELDS)
 
 All arithmetic runs in libftgp.so (hand-written sm_100a CUDA behind include/ftgp.h); torch only
 owns the device memory and the stream.  There is no CPU fallback: constructing a Fleet without a
@@ -24,12 +26,13 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import (DRIVER_FAST, DRIVER_LOBOTOMY, DRIVER_NIDC, LAP_FIELDS, MAX_LAPTIMES, NBEAMS, NQ, NU, NV)
+from ._lib import (DRIVER_FAST, DRIVER_LOBOTOMY, DRIVER_NIDC, LAP_FIELDS, MAX_LAPTIMES, NBEAMS, NQ, NU, NV, RACE_FIELDS)
 from .track import Geometry, Track
 from .vehicle import VehicleStateSnapshot
 
 TIMESTEP = 0.004                      # template/mushr.em.xml:30
 LAP = {name: k for k, name in enumerate(LAP_FIELDS)}
+RACE = {name: k for k, name in enumerate(RACE_FIELDS)}
 DRIVER_KINDS = {"nidc": DRIVER_NIDC, "fast": DRIVER_FAST, "lobotomy": DRIVER_LOBOTOMY,
                 "ft_grandprix.nidc": DRIVER_NIDC, "ft_grandprix.fast": DRIVER_FAST,
                 "ft_grandprix.lobotomy": DRIVER_LOBOTOMY}
@@ -39,8 +42,12 @@ def _ptr(t):
 
 class Fleet:
     def __init__(self, tracks, ncars, cars_per_world=1, device=0, track_id=None, driver="nidc",
-                 lap_target=10, naive_flatten=False, bubble_wrap=False):
-        """lap_target, naive_flatten, bubble_wrap: the path-relevant options of the reference (custom.py:961,981,970)."""
+                 lap_target=10, naive_flatten=False, bubble_wrap=False, reload_finished=False, race_ticks=0):
+        """lap_target, naive_flatten, bubble_wrap: the path-relevant options of the reference (custom.py:961,981,970).
+        reload_finished: race after race on the device.  At the head of every tick a world whose cars have all finished,
+        or whose race has run race_ticks ticks (race_ticks > 0), is reloaded (custom.py:1089-1128) from the next-start
+        tensors (set_next_start(); by default the poses of the last reset()), and the race that ended is added to
+        race_tally[car] (RACE fields).  The other worlds go on racing."""
         if not torch.cuda.is_available():
             raise _lib.FtgpError("Fleet needs a CUDA device (sm_100a); there is no CPU fallback")
         self.lib = _lib.load()
@@ -51,6 +58,10 @@ class Fleet:
             raise ValueError("ncars must be a multiple of cars_per_world")
         self.nworlds = self.ncars // self.cars_per_world
         self.lap_target = int(lap_target)
+        self.reload_finished = bool(reload_finished)
+        self.race_ticks = int(race_ticks)
+        if self.race_ticks < 0:
+            raise ValueError("race_ticks must be >= 0")
         self.naive_flatten = bool(naive_flatten)
         self.bubble_wrap = bool(bubble_wrap)
         self.default_driver = DRIVER_KINDS[driver] if isinstance(driver, str) else int(driver)
@@ -69,6 +80,12 @@ class Fleet:
         self.track_id = None if track_id is None else torch.as_tensor(track_id, dtype=torch.int32).to(dev).contiguous()
         self.driver_kind = None
         self.steps = 0
+        if self.reload_finished:
+            self.race_tally = torch.zeros(n, len(RACE_FIELDS), dtype=torch.int32, device=dev)
+            self.race_start = torch.zeros(self.nworlds, dtype=torch.int32, device=dev)   # tick at which the world's race began
+            self.start_xy = torch.zeros(n, 2, dtype=torch.float64, device=dev)           # the next race's start grid
+            self.start_yaw = torch.zeros(n, dtype=torch.float64, device=dev)
+            self.start_offset = self._grid_offsets()
         # options manual_control / always_invoke_driver / detach_control of the loop's driver block (custom.py:952-957,1401-1423)
         self.manual_control = False          # the watched car takes (speed, steering) from the operator
         self.always_invoke_driver = True     # ... while the drivers are still invoked (reference default)
@@ -108,6 +125,11 @@ class Fleet:
         k = [DRIVER_KINDS[x] if isinstance(x, str) else int(x) for x in kinds]
         self.driver_kind = torch.tensor(k, dtype=torch.int32, device=self.device)
 
+    def _grid_offsets(self):
+        """VehicleState(offset=(i+5)*2) of grid slot i (custom.py:96-118)."""
+        idx = torch.arange(self.ncars, device=self.device, dtype=torch.int32) % self.cars_per_world
+        return (idx + 5) * 2
+
     # ------------------------------------------------------------------ reset (custom.py:1089-1128,1232-1245)
     def reset(self, xy, yaw):
         xy = torch.as_tensor(np.asarray(xy, dtype=np.float64)).to(self.device).contiguous()
@@ -120,9 +142,12 @@ class Fleet:
         with torch.cuda.stream(self.stream):
             self.ranges.zero_(); self.lap.zero_(); self.times.zero_(); self.winners.zero_(); self.status.zero_()
             # VehicleState(offset=(i+5)*2) with good_start=True (custom.py:96-118)
-            idx = torch.arange(self.ncars, device=self.device, dtype=torch.int32) % self.cars_per_world
-            self.lap[:, LAP["offset"]] = (idx + 5) * 2
+            self.lap[:, LAP["offset"]] = self._grid_offsets()
             self.lap[:, LAP["good_start"]] = 1
+            if self.reload_finished:                  # the default next start; a reset begins a new series
+                self.start_xy.copy_(xy); self.start_yaw.copy_(yaw)
+                self.start_offset.copy_(self.lap[:, LAP["offset"]])
+                self.race_start.zero_(); self.race_tally.zero_()
         self.steps = 0
         self.sync()
         self._keep = (xy, yaw)
@@ -137,6 +162,43 @@ class Fleet:
             sel = tid == k
             xy[sel] = poses[slot[sel], :2]; yaw[sel] = poses[slot[sel], 2]
         self.reset(xy, yaw)
+
+    # ------------------------------------------------------------------ race after race (reload_finished)
+    def set_next_start(self, xy, yaw, offset=None):
+        """Start poses ([ncars, 2], [ncars]) and lap offsets ([ncars]; default: the grid slot's (slot+5)*2, as reset()
+        sets it) of the next race of every world.  They are read when a world is reloaded, so a caller may rewrite them
+        between ticks, e.g. grid poses plus seeded jitter: device drivers are deterministic, and a world reloaded from an
+        unchanged start runs the same race again."""
+        self._need_reload("set_next_start")
+        xy = torch.as_tensor(xy, dtype=torch.float64, device=self.device)
+        yaw = torch.as_tensor(yaw, dtype=torch.float64, device=self.device)
+        off = self._grid_offsets() if offset is None else torch.as_tensor(offset, dtype=torch.int32, device=self.device)
+        if xy.shape != (self.ncars, 2) or yaw.shape != (self.ncars,) or off.shape != (self.ncars,):
+            raise ValueError("xy must be [ncars,2], yaw and offset [ncars]")
+        self.stream.wait_stream(torch.cuda.current_stream(self.device))
+        with torch.cuda.stream(self.stream):            # in stream order: ticks already issued read the old starts
+            self.start_xy.copy_(xy); self.start_yaw.copy_(yaw); self.start_offset.copy_(off)
+        for t in (xy, yaw, off):
+            t.record_stream(self.stream)
+
+    def _need_reload(self, what):
+        if not self.reload_finished:
+            raise ValueError(f"{what} needs Fleet(..., reload_finished=True)")
+
+    def reload_args(self):
+        self._need_reload("reload_args")
+        r = _lib.ReloadArgs()
+        r.start_xy, r.start_yaw, r.start_offset = (self.start_xy.data_ptr(), self.start_yaw.data_ptr(),
+                                                   self.start_offset.data_ptr())
+        r.race_start, r.tally = self.race_start.data_ptr(), self.race_tally.data_ptr()
+        r.race_ticks = self.race_ticks
+        return r
+
+    def reload(self):
+        """Reload the worlds whose race is over, now (the piece fleet.tick() runs at the head of every tick, for loops
+        that issue the tick's pieces one by one: reload -> lap_update -> drive -> lidar -> step)."""
+        a, r = self.tick_args(), self.reload_args()
+        _lib.check(self.lib.ftgp_reload(C.byref(a), C.byref(r), self._s), "ftgp_reload")
 
     # ------------------------------------------------------------------ the per-tick pieces
     def lidar(self, visible=None, min_range=None, shadow_finished=True, qpos=None, stream=None):
@@ -273,10 +335,16 @@ class Fleet:
         """nticks iterations of the physics loop (custom.py:1337-1426), all on device."""
         if self._control_options():                   # operator options: the driver block needs the host's say every tick
             for _ in range(int(nticks)):
+                if self.reload_finished:
+                    self.reload()
                 self.lap_update(); self.drive(); self.lidar(); self.step(1)
             return
         a = self.tick_args()
-        _lib.check(self.lib.ftgp_tick(C.byref(a), int(nticks), self._s), "ftgp_tick")
+        if self.reload_finished:
+            r = self.reload_args()
+            _lib.check(self.lib.ftgp_tick_reload(C.byref(a), C.byref(r), int(nticks), self._s), "ftgp_tick_reload")
+        else:
+            _lib.check(self.lib.ftgp_tick(C.byref(a), int(nticks), self._s), "ftgp_tick")
         self.steps += int(nticks)
 
     def tick_readback(self, ranges_host, lap_host, cars=None):
@@ -297,6 +365,9 @@ class Fleet:
         lap_ready, ranges_ready, lap_copied, ranges_copied, poses_copied = self._ev
         with torch.cuda.stream(s):
             s.wait_event(lap_copied)                 # the previous copy of the lap state has left
+            if self.reload_finished:
+                s.wait_event(ranges_copied)          # ... and of the ranges: a reload writes both
+                self.reload()
             self.lap_update()
             lap_ready.record(s)
             self.drive()
@@ -367,12 +438,17 @@ class Fleet:
                     "lap_completion": lap_completion, "absolute_completion": laps * 100 + lap_completion,
                     "time": self.steps / TIMESTEP}                                            # custom.py:1397 (sic)
 
+    def _state_keys(self):
+        keys = ("qpos", "qvel", "warm", "ctrl", "ranges", "lap", "times", "winners", "status")
+        if self.reload_finished:
+            keys += ("race_tally", "race_start", "start_xy", "start_yaw", "start_offset")
+        return keys
+
     def state_dict(self):
         self.sync()
-        return {k: getattr(self, k).cpu() for k in ("qpos", "qvel", "warm", "ctrl", "ranges", "lap", "times",
-                                                     "winners", "status")} | {"steps": self.steps}
+        return {k: getattr(self, k).cpu() for k in self._state_keys()} | {"steps": self.steps}
 
     def load_state_dict(self, sd):
-        for k in ("qpos", "qvel", "warm", "ctrl", "ranges", "lap", "times", "winners", "status"):
+        for k in self._state_keys():
             getattr(self, k).copy_(sd[k])
         self.steps = int(sd["steps"])

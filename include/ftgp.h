@@ -190,6 +190,36 @@ int ftgp_naive_flatten(double* qpos, int64_t qpos_stride, int64_t ncars, void* s
  * lives in a device counter).  ftgp_release_graphs() drops the cached graphs. */
 int ftgp_tick(const ftgp_tick_args* a, int nticks, void* stream);
 int ftgp_release_graphs(void);
+
+/* ------------------------------------------------------------------ race after race (reload(), custom.py:1089-1128) */
+/* A world is due at the head of a tick when every one of its cars has FTGP_LAP_FINISHED set, or when race_ticks > 0 and
+ * steps - race_start[w] >= race_ticks.  A due world is reloaded before anything else of the tick runs: the race that
+ * just ended is added to its cars' tally rows, then its cars are reset exactly as ftgp_reset + a fresh lap state would
+ * leave them (qpos / qvel / warm / ctrl from start_xy / start_yaw; ranges, times, status and the lap row zero except
+ * FTGP_LAP_OFFSET = start_offset, FTGP_LAP_GOOD_START = 1, FTGP_LAP_START = steps), winners[w] = 0 and
+ * race_start[w] = steps.  `steps` is the value the lap update of the same tick sees.  Worlds that are not due are not
+ * written.  The start tensors are read when a world is reloaded; the caller may rewrite them between calls. */
+enum {
+    FTGP_RACE_RACES = 0, FTGP_RACE_FINISHED, FTGP_RACE_WINS, FTGP_RACE_RANK_SUM, FTGP_RACE_LAPS_SUM,
+    FTGP_RACE_TIME_SUM, FTGP_RACE_BEST_LAP, FTGP_RACE_OFFTRACK_TICKS, FTGP_RACE_CONTACT_TICKS, FTGP_RACE_FIELDS
+};
+/* Per car and race: RACES += 1; FINISHED += finished; WINS += rank == 1; RANK_SUM += rank (0 = did not finish);
+ * LAPS_SUM += laps; TIME_SUM += the stored lap times (times[0 : min(ntimes, 16)]) of a finished car (run.py:78);
+ * BEST_LAP = min(BEST_LAP, stored lap times), 0 = no lap recorded yet; OFFTRACK_TICKS / CONTACT_TICKS += the lap
+ * state's FTGP_LAP_OFFTRACK_TICKS / FTGP_LAP_CONTACT_TICKS. */
+typedef struct {
+    const double* start_xy;      /* device double[ncars][2]  pose of the next race (custom.py:1232-1245) */
+    const double* start_yaw;     /* device double[ncars] */
+    const int32_t* start_offset; /* device int32[ncars]      FTGP_LAP_OFFSET of the next race */
+    int32_t* race_start;         /* device int32[nworlds]    tick at which the world's current race began, or NULL */
+    int32_t* tally;              /* device int32[ncars][FTGP_RACE_FIELDS] or NULL (needs race_start) */
+    int32_t race_ticks;          /* 0 = a world is due only when all its cars have finished (> 0 needs race_start) */
+    int32_t reserved;
+} ftgp_reload_args;
+/* Un-fused: reload the due worlds now, with steps = a->steps (for loops that issue the tick's pieces one by one). */
+int ftgp_reload(const ftgp_tick_args* a, const ftgp_reload_args* r, void* stream);
+/* ftgp_tick with the reload at the head of every tick (graph-replayed like ftgp_tick); r == NULL is exactly ftgp_tick. */
+int ftgp_tick_reload(const ftgp_tick_args* a, const ftgp_reload_args* r, int nticks, void* stream);
 /* enable != 0 (default): small fleets replay the captured tick; 0: every tick is issued launch by launch.
  * Returns the previous setting (for A/B timing in the bench). */
 int ftgp_tick_use_graphs(int enable);
