@@ -16,6 +16,8 @@ LAP_FIELDS = ("offset", "completion", "laps", "start", "good_start", "finished",
 RACE_FIELDS = ("races", "finished", "wins", "rank_sum", "laps_sum", "time_sum", "best_lap", "offtrack_ticks",
                "contact_ticks")
 DRIVER_NIDC, DRIVER_FAST, DRIVER_LOBOTOMY = 0, 1, 2
+DRV_FIELDS = ("car_width", "safety_percentage", "difference_threshold", "speed", "speed_divisor", "max_steer",
+              "boost_speed", "boost_max_steer", "boost_min_rear_range", "speed_cap")
 OPT_NAIVE_FLATTEN, OPT_BUBBLE_WRAP = 1, 2
 
 class FtgpError(RuntimeError):
@@ -58,12 +60,14 @@ SIGNATURES = {
     "ftgp_release_scratch": (_i, [_vp]),
     "ftgp_naive_flatten": (_i, [_vp, _i64, _i64, _vp]),
     "ftgp_drivers": (_i, [_vp, _vp, _i, _vp, _vp, _i64, _vp]),
+    "ftgp_drivers_params": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _i64, _vp]),
     "ftgp_lap_update": (_i, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _i64, _i, C.c_int32, C.c_int32, _vp]),
     "ftgp_tick": (_i, [C.POINTER(TickArgs), _i, _vp]),
     "ftgp_release_graphs": (_i, []),
     "ftgp_tick_use_graphs": (_i, [_i]),
     "ftgp_reload": (_i, [C.POINTER(TickArgs), C.POINTER(ReloadArgs), _vp]),
     "ftgp_tick_reload": (_i, [C.POINTER(TickArgs), C.POINTER(ReloadArgs), _i, _vp]),
+    "ftgp_tick_params": (_i, [C.POINTER(TickArgs), C.POINTER(ReloadArgs), _vp, _i, _vp]),
 }
 
 _lib = None

@@ -143,9 +143,31 @@ __device__ __forceinline__ double pick(double e0, double e1, double e2, int idx)
     return __shfl_sync(0xffffffffu, v, idx & 31);
 }
 
+// Field F of the reference row of a bundled kind (include/ftgp.h FTGP_DRV_*), folded at compile time.
+__device__ __forceinline__ double default_field(bool nidc, int f) {
+    const double PI = 3.141592653589793;
+    switch (f) {
+    case FTGP_DRV_CAR_WIDTH:            return nidc ? 0.12 : 0.06;               // nidc.py:5, fast.py:4
+    case FTGP_DRV_SAFETY_PERCENTAGE:    return 300.;                             // nidc.py:10
+    case FTGP_DRV_DIFFERENCE_THRESHOLD: return 0.6;                              // nidc.py:7
+    case FTGP_DRV_SPEED:                return 0.5;                              // nidc.py:8
+    case FTGP_DRV_SPEED_DIVISOR:        return nidc ? 1.57 * 2 : PI;             // nidc.py:130, fast.py:138
+    case FTGP_DRV_MAX_STEER:            return 90.0 * (PI / 180.0);              // nidc.py:113
+    case FTGP_DRV_BOOST_SPEED:          return 7;                                // fast.py:136
+    case FTGP_DRV_BOOST_MAX_STEER:      return nidc ? 0.0 : 0.1;                 // fast.py:135 (nidc: never)
+    case FTGP_DRV_BOOST_MIN_REAR_RANGE: return 0.5;                              // fast.py:135
+    default:                            return nidc ? INFINITY : 2.0;            // fast.py:138 SPEED_CAP
+    }
+}
+// the car's row (lane-uniform address: one broadcast load per field), or its kind's reference row
+template <int F> __device__ __forceinline__ double drv(const double* __restrict__ row, int k) {
+    return row ? row[F] : default_field(k == FTGP_DRIVER_NIDC, F);
+}
+
 __global__ void __launch_bounds__(256)
 drivers_kernel(const float* __restrict__ ranges, const int32_t* __restrict__ kind, int default_kind,
-               const int32_t* __restrict__ lap, double* __restrict__ ctrl, int64_t ncars, int32_t* __restrict__ steps_dev) {
+               const double* __restrict__ params, const int32_t* __restrict__ lap, double* __restrict__ ctrl, int64_t ncars,
+               int32_t* __restrict__ steps_dev) {
     const int lane = threadIdx.x & 31;
     const int64_t car = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     // graph-replayed tick: the lap kernel (earlier on this stream) has read the tick counter; nothing else reads it this tick
@@ -155,6 +177,7 @@ drivers_kernel(const float* __restrict__ ranges, const int32_t* __restrict__ kin
     if (lap && lap[car * FTGP_LAP_FIELDS + FTGP_LAP_FINISHED]) k = FTGP_DRIVER_LOBOTOMY;   // shadow(): custom.py:1437
     double* out = ctrl + 2 * car;
     if (k == FTGP_DRIVER_LOBOTOMY) { if (lane == 0) { out[0] = 0.0; out[1] = 0.0; } return; }
+    const double* prow = params ? params + car * FTGP_DRV_FIELDS : nullptr;
     const float* row = ranges + car * FTGP_NBEAMS;
     const double PI = 3.141592653589793;
     const double rpp = (2 * PI) / FTGP_NBEAMS;                  // nidc.py:121
@@ -163,16 +186,17 @@ drivers_kernel(const float* __restrict__ ranges, const int32_t* __restrict__ kin
     double e1 = (double)row[EIGHTH + 32 + lane];
     double e2 = lane < NPROC - 64 ? (double)row[EIGHTH + 64 + lane] : 0.0;
     const float r0 = row[0];
-    // disparities from the unmodified array (nidc.py:123-124): |proc[i] - proc[i-1]| > 0.6, i >= 1
+    // disparities from the unmodified array (nidc.py:123-124): |proc[i] - proc[i-1]| > threshold, i >= 1
+    const double thr = drv<FTGP_DRV_DIFFERENCE_THRESHOLD>(prow, k);
     double p0 = __shfl_up_sync(0xffffffffu, e0, 1);
     double l0 = __shfl_sync(0xffffffffu, e0, 31), l1 = __shfl_sync(0xffffffffu, e1, 31);
     double p1 = __shfl_up_sync(0xffffffffu, e1, 1); if (lane == 0) p1 = l0;
     double p2 = __shfl_up_sync(0xffffffffu, e2, 1); if (lane == 0) p2 = l1;
-    unsigned m0 = __ballot_sync(0xffffffffu, lane > 0 && fabs(e0 - p0) > 0.6);
-    unsigned m1 = __ballot_sync(0xffffffffu, fabs(e1 - p1) > 0.6);
-    unsigned m2 = __ballot_sync(0xffffffffu, lane < NPROC - 64 && fabs(e2 - p2) > 0.6);
-    const double car_width = k == FTGP_DRIVER_NIDC ? 0.12 : 0.06;     // nidc.py:5, fast.py:4
-    const double width = (car_width / 2) * (1 + 300. / 100);          // nidc.py:93
+    unsigned m0 = __ballot_sync(0xffffffffu, lane > 0 && fabs(e0 - p0) > thr);
+    unsigned m1 = __ballot_sync(0xffffffffu, fabs(e1 - p1) > thr);
+    unsigned m2 = __ballot_sync(0xffffffffu, lane < NPROC - 64 && fabs(e2 - p2) > thr);
+    // nidc.py:93; with the reference rows this equals the constant the literals fold to, bit for bit
+    const double width = (drv<FTGP_DRV_CAR_WIDTH>(prow, k) / 2) * (1 + drv<FTGP_DRV_SAFETY_PERCENTAGE>(prow, k) / 100);
     bool raised = false;
     for (int seg = 0; seg < 3 && !raised; seg++) {
         unsigned m = seg == 0 ? m0 : (seg == 1 ? m1 : m2);
@@ -222,12 +246,16 @@ drivers_kernel(const float* __restrict__ ranges, const int32_t* __restrict__ kin
     }
     if (lane == 0) {
         double ang = ((double)bi - (NPROC / 2.0)) * rpp;              // nidc.py:112
-        const double lim = 90.0 * (PI / 180.0);
+        const double lim = drv<FTGP_DRV_MAX_STEER>(prow, k);          // nidc.py:113
         double st = ang < -lim ? -lim : (ang > lim ? lim : ang);
         double sp;
-        if (k == FTGP_DRIVER_NIDC) sp = 0.5 * 5 * (1 - fabs(st) / (1.57 * 2));      // nidc.py:130
-        else if (fabs(st) < 0.1 && (double)r0 > 0.5) sp = 7;                          // fast.py:135-136
-        else { double s = 0.5 * 5 * (1 - fabs(st) / PI); sp = s < 2 ? s : 2; }      // fast.py:138
+        if (fabs(st) < drv<FTGP_DRV_BOOST_MAX_STEER>(prow, k) && (double)r0 > drv<FTGP_DRV_BOOST_MIN_REAR_RANGE>(prow, k))
+            sp = drv<FTGP_DRV_BOOST_SPEED>(prow, k);                                        // fast.py:135-136
+        else {                                                                              // nidc.py:130, fast.py:138
+            const double s = drv<FTGP_DRV_SPEED>(prow, k) * 5 * (1 - fabs(st) / drv<FTGP_DRV_SPEED_DIVISOR>(prow, k));
+            const double cap = drv<FTGP_DRV_SPEED_CAP>(prow, k);
+            sp = s < cap ? s : cap;
+        }
         out[0] = sp; out[1] = st;                                      // custom.py:1422-1423
     }
 }
@@ -292,11 +320,11 @@ __global__ void lap_kernel(const uint32_t* __restrict__ blob, const double* __re
     if (winners) winners[world] = nwin;
 }
 
-int launch_drivers(const float* ranges, const int32_t* kind, int default_kind, const int32_t* lap, double* ctrl,
-                   int64_t ncars, cudaStream_t stream, int32_t* steps_dev) {
+int launch_drivers(const float* ranges, const int32_t* kind, int default_kind, const double* params, const int32_t* lap,
+                   double* ctrl, int64_t ncars, cudaStream_t stream, int32_t* steps_dev) {
     const int threads = 256;
     int64_t blocks = (ncars * 32 + threads - 1) / threads;
-    drivers_kernel<<<(unsigned)blocks, threads, 0, stream>>>(ranges, kind, default_kind, lap, ctrl, ncars, steps_dev);
+    drivers_kernel<<<(unsigned)blocks, threads, 0, stream>>>(ranges, kind, default_kind, params, lap, ctrl, ncars, steps_dev);
     count_launch();
     FTGP_CUDA(cudaGetLastError());
     return FTGP_OK;
@@ -333,11 +361,16 @@ extern "C" int ftgp_naive_flatten(double* qpos, int64_t qpos_stride, int64_t nca
     return launch_flatten(qpos, qpos_stride, ncars, (cudaStream_t)stream);
 }
 
-extern "C" int ftgp_drivers(const float* ranges, const int32_t* kind, int default_kind, const int32_t* lap,
-                            double* ctrl, int64_t ncars, void* stream) {
+extern "C" int ftgp_drivers_params(const float* ranges, const int32_t* kind, int default_kind, const double* params,
+                                   const int32_t* lap, double* ctrl, int64_t ncars, void* stream) {
     if (!ranges || !ctrl || ncars < 0 || default_kind < 0 || default_kind > 2) { set_error("ftgp_drivers: bad argument"); return FTGP_ERR_ARG; }
     if (ncars == 0) return FTGP_OK;
-    return launch_drivers(ranges, kind, default_kind, lap, ctrl, ncars, (cudaStream_t)stream, nullptr);
+    return launch_drivers(ranges, kind, default_kind, params, lap, ctrl, ncars, (cudaStream_t)stream, nullptr);
+}
+
+extern "C" int ftgp_drivers(const float* ranges, const int32_t* kind, int default_kind, const int32_t* lap,
+                            double* ctrl, int64_t ncars, void* stream) {
+    return ftgp_drivers_params(ranges, kind, default_kind, nullptr, lap, ctrl, ncars, stream);
 }
 
 extern "C" int ftgp_lap_update(const ftgp_geom* g, const double* qpos, int64_t qpos_stride,

@@ -457,8 +457,8 @@ int launch_step(const ftgp_geom* g, double* qpos, double* qvel, double* warm, co
 int launch_lidar(const ftgp_geom* g, const double* qpos, int64_t stride, const int32_t* track_id,
                  const uint8_t* visible, const int32_t* lap, int64_t ncars, int cpw, float* ranges, float* min_range,
                  cudaStream_t stream);
-int launch_drivers(const float* ranges, const int32_t* kind, int default_kind, const int32_t* lap, double* ctrl,
-                   int64_t ncars, cudaStream_t stream, int32_t* steps_dev);
+int launch_drivers(const float* ranges, const int32_t* kind, int default_kind, const double* params, const int32_t* lap,
+                   double* ctrl, int64_t ncars, cudaStream_t stream, int32_t* steps_dev);
 int launch_lap(const ftgp_geom* g, const double* qpos, int64_t stride, const int32_t* track_id, int32_t* lap,
                int32_t* times, int32_t* winners, const int32_t* status, int64_t ncars, int cpw, int32_t steps,
                int32_t lap_target, cudaStream_t stream, const int32_t* steps_dev);
@@ -499,8 +499,9 @@ static int overlap_fork(double* qpos, int64_t ncars, bool copy, cudaStream_t str
 }
 
 // ---- one tick = custom.py:1337-1426 for the whole fleet, in the reference's order; r != NULL: the worlds whose race is
-// over are reloaded first (custom.py:1089-1128)
-static int issue_tick(const ftgp_tick_args* a, const ftgp_reload_args* r, int32_t steps, int32_t* steps_dev, cudaStream_t s) {
+// over are reloaded first (custom.py:1089-1128); dp != NULL: the drivers read the per-car rows (ftgp_drivers_params)
+static int issue_tick(const ftgp_tick_args* a, const ftgp_reload_args* r, const double* dp, int32_t steps, int32_t* steps_dev,
+                      cudaStream_t s) {
     int rc;
     if (r && (rc = launch_reload(a, r, steps, s, steps_dev))) return rc;
     // custom.py:1338-1339 option naive_flatten
@@ -509,7 +510,7 @@ static int issue_tick(const ftgp_tick_args* a, const ftgp_reload_args* r, int32_
     if ((rc = launch_lap(a->geom, a->qpos, FTGP_NQ, a->track_id, a->lap, a->times, a->winners, a->status, a->ncars,
                          a->cars_per_world, steps, a->lap_target, s, steps_dev))) return rc;
     // custom.py:1395-1423 driver on the ranges of the previous mj_step, control write
-    if ((rc = launch_drivers(a->ranges, a->driver_kind, a->default_driver, a->lap, a->ctrl, a->ncars, s, steps_dev))) return rc;
+    if ((rc = launch_drivers(a->ranges, a->driver_kind, a->default_driver, dp, a->lap, a->ctrl, a->ncars, s, steps_dev))) return rc;
     // custom.py:1425 mj_step: rangefinders are evaluated from the pre-step pose, then the state advances.  The rangefinder
     // kernel scans a copy of the poses on a stream of its own beside the step; in worlds of several cars the coupled worlds'
     // solver starts here as well, on a third stream (launch_worlds_early takes the copy in that case).
@@ -531,7 +532,8 @@ static int issue_tick(const ftgp_tick_args* a, const ftgp_reload_args* r, int32_
 constexpr int64_t GRAPH_MAX_CARS = 16384;
 static std::atomic<int> g_use_graphs{1};
 struct TickGraph {
-    ftgp_tick_args key{}; bool reload = false; ftgp_reload_args rkey{}; cudaStream_t stream = nullptr; int dev = -1;
+    ftgp_tick_args key{}; bool reload = false; ftgp_reload_args rkey{}; const double* params = nullptr;
+    cudaStream_t stream = nullptr; int dev = -1;
     cudaGraphExec_t exec = nullptr; int32_t* steps_dev = nullptr; int32_t shadow = INT32_MIN;
     uint64_t scratch_gen = 0; int launches_per_tick = 0; bool seen = false; uint64_t used = 0;
 };
@@ -564,14 +566,16 @@ static void drop_graph(TickGraph& g) {
 }
 
 // returns FTGP_OK and sets *done = number of ticks issued through the graph (0: caller runs them eagerly)
-static int graph_ticks(const ftgp_tick_args* a, const ftgp_reload_args* r, int nticks, cudaStream_t s, int* done) {
+static int graph_ticks(const ftgp_tick_args* a, const ftgp_reload_args* r, const double* dp, int nticks, cudaStream_t s,
+                       int* done) {
     *done = 0;
     int dev = 0;
     FTGP_CUDA(cudaGetDevice(&dev));
     std::lock_guard<std::mutex> lock(g_graph_mutex);
     TickGraph* e = nullptr; TickGraph* lru = &g_graphs[0];
     for (auto& g : g_graphs) {
-        if (g.seen && g.dev == dev && g.stream == s && same_key(g.key, *a) && same_reload(g, r)) { e = &g; break; }
+        if (g.seen && g.dev == dev && g.stream == s && same_key(g.key, *a) && same_reload(g, r) &&
+            g.params == dp) { e = &g; break; }
         if (g.used < lru->used) lru = &g;
     }
     int32_t steps = a->steps;
@@ -580,8 +584,9 @@ static int graph_ticks(const ftgp_tick_args* a, const ftgp_reload_args* r, int n
         lru->key = *a; lru->stream = s; lru->dev = dev; lru->seen = true;
         lru->reload = r != nullptr;
         if (r) lru->rkey = *r;
+        lru->params = dp;
         e = lru;
-        const int rc = issue_tick(a, r, steps, nullptr, s);
+        const int rc = issue_tick(a, r, dp, steps, nullptr, s);
         if (rc) return rc;
         steps++; nticks--; *done = 1;
         if (nticks == 0) { e->used = ++g_graph_clock; return FTGP_OK; }
@@ -594,7 +599,7 @@ static int graph_ticks(const ftgp_tick_args* a, const ftgp_reload_args* r, int n
         const int64_t l0 = ftgp_launch_count();
         cudaGraph_t graph = nullptr;
         FTGP_CUDA(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-        const int rc = issue_tick(a, r, 0, e->steps_dev, s);
+        const int rc = issue_tick(a, r, dp, 0, e->steps_dev, s);
         const cudaError_t ce = cudaStreamEndCapture(s, &graph);
         if (rc || ce != cudaSuccess || !graph) {                 // capture refused (e.g. scratch had to grow): stay eager
             if (graph) cudaGraphDestroy(graph);
@@ -649,7 +654,8 @@ static bool bad_reload_args(const ftgp_reload_args* r) {
            (r->tally && !r->race_start) || (r->race_ticks > 0 && !r->race_start);
 }
 
-extern "C" int ftgp_tick_reload(const ftgp_tick_args* a, const ftgp_reload_args* r, int nticks, void* stream) {
+extern "C" int ftgp_tick_params(const ftgp_tick_args* a, const ftgp_reload_args* r, const double* driver_params, int nticks,
+                                void* stream) {
     if (bad_tick_args(a) || nticks < 0) { set_error("ftgp_tick: bad argument"); return FTGP_ERR_ARG; }
     if (r && bad_reload_args(r)) { set_error("ftgp_tick_reload: bad reload argument"); return FTGP_ERR_ARG; }
     if (a->ncars == 0 || nticks == 0) return FTGP_OK;
@@ -657,11 +663,15 @@ extern "C" int ftgp_tick_reload(const ftgp_tick_args* a, const ftgp_reload_args*
     cudaStream_t s = (cudaStream_t)stream;
     int t0 = 0, rc;
     if (a->ncars <= GRAPH_MAX_CARS && s != nullptr && g_use_graphs.load()) {           // (the legacy default stream cannot be captured)
-        if ((rc = graph_ticks(a, r, nticks, s, &t0))) return rc;
+        if ((rc = graph_ticks(a, r, driver_params, nticks, s, &t0))) return rc;
     }
     for (int t = t0; t < nticks; t++)
-        if ((rc = issue_tick(a, r, a->steps + t, nullptr, s))) return rc;
+        if ((rc = issue_tick(a, r, driver_params, a->steps + t, nullptr, s))) return rc;
     return FTGP_OK;
+}
+
+extern "C" int ftgp_tick_reload(const ftgp_tick_args* a, const ftgp_reload_args* r, int nticks, void* stream) {
+    return ftgp_tick_params(a, r, nullptr, nticks, stream);
 }
 
 extern "C" int ftgp_tick(const ftgp_tick_args* a, int nticks, void* stream) { return ftgp_tick_reload(a, nullptr, nticks, stream); }

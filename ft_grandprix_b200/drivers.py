@@ -33,12 +33,37 @@ class BatchedLobotomyDriver:
 
 
 class BatchedNidcDriver:
+    """The class constants are the reference row (include/ftgp.h FTGP_DRV_*, names in _lib.DRV_FIELDS); `params`, a
+    float64 tensor [n, 10] of such rows, overrides them per scan.  With rows, each row alone decides its driver (the
+    class no longer matters), as in Fleet.set_driver_params()."""
     CAR_WIDTH = 0.12                 # nidc.py:5
+    SAFETY_PERCENTAGE = 300.         # nidc.py:10
     DIFFERENCE_THRESHOLD = 0.6       # nidc.py:7
     SPEED = 0.5                      # nidc.py:8
-    SAFETY_PERCENTAGE = 300.         # nidc.py:10
+    SPEED_DIVISOR = 1.57 * 2         # nidc.py:130
+    MAX_STEER = math.radians(90)     # nidc.py:113
+    BOOST_SPEED = 7.0                # fast.py:136
+    BOOST_MAX_STEER = 0.0            # fast.py:135 (|st| < 0 never holds: no boost)
+    BOOST_MIN_REAR_RANGE = 0.5       # fast.py:135
+    SPEED_CAP = math.inf             # fast.py:138 (no cap)
 
-    def _extend(self, ranges):
+    def __init__(self, params=None):
+        self.params = params
+
+    @classmethod
+    def default_row(cls):
+        from ._lib import DRV_FIELDS
+        return [float(getattr(cls, name.upper())) for name in DRV_FIELDS]
+
+    def _rows(self, n, device):
+        if self.params is None:
+            return torch.tensor(self.default_row(), dtype=torch.float64, device=device).expand(n, -1)
+        p = torch.as_tensor(self.params, dtype=torch.float64, device=device)
+        if p.shape != (n, 10):
+            raise ValueError(f"params must be [{n}, 10]")
+        return p
+
+    def _extend(self, ranges, p):
         r = ranges.to(torch.float64)
         n, nb = r.shape
         rpp = (2 * math.pi) / nb                                     # nidc.py:121
@@ -47,8 +72,8 @@ class BatchedNidcDriver:
         m = proc.shape[1]
         diff = torch.zeros_like(proc)
         diff[:, 1:] = (proc[:, 1:] - proc[:, :-1]).abs()             # nidc.py:26-29
-        disp = diff > self.DIFFERENCE_THRESHOLD                      # nidc.py:31-40 (computed once)
-        width = (self.CAR_WIDTH / 2) * (1 + self.SAFETY_PERCENTAGE / 100)   # nidc.py:93
+        disp = diff > p[:, 2:3]                                      # nidc.py:31-40 (computed once)
+        width = (p[:, 0] / 2) * (1 + p[:, 1] / 100)                  # nidc.py:93
         idx = torch.arange(m, device=r.device).unsqueeze(0)          # [1, m]
         raised = torch.zeros(n, dtype=torch.bool, device=r.device)
         for i in range(1, m):                                        # nidc.py:94-104, in index order
@@ -76,22 +101,23 @@ class BatchedNidcDriver:
         first_max = (torch.nan_to_num(proc, nan=-math.inf) == mx).float().argmax(1)
         best = torch.where(nan_any, first_nan, first_max)
         ang = (best.to(torch.float64) - m / 2.0) * rpp               # nidc.py:112
-        steer = ang.clamp(-math.radians(90), math.radians(90))       # nidc.py:113
+        lim = p[:, 5]                                                # nidc.py:113
+        steer = torch.where(ang < -lim, -lim, torch.where(ang > lim, lim, ang))
         return steer, raised, r
 
     def process_lidar(self, ranges):
-        steer, raised, _ = self._extend(ranges)
-        speed = self.SPEED * 5 * (1 - steer.abs() / (1.57 * 2))      # nidc.py:130
+        p = self._rows(ranges.shape[0], ranges.device)
+        steer, raised, r = self._extend(ranges, p)
+        s = p[:, 3] * 5 * (1 - steer.abs() / p[:, 4])                # nidc.py:130, fast.py:138
+        slow = torch.where(s < p[:, 9], s, p[:, 9])
+        boost = (steer.abs() < p[:, 7]) & (r[:, 0] > p[:, 8])        # fast.py:135-136
+        speed = torch.where(boost, p[:, 6], slow)
         self.raised = raised
         return speed, steer
 
 
 class BatchedFastDriver(BatchedNidcDriver):
     CAR_WIDTH = 0.06                 # fast.py:4
-
-    def process_lidar(self, ranges):
-        steer, raised, r = self._extend(ranges)
-        slow = torch.clamp(self.SPEED * 5 * (1 - steer.abs() / math.pi), max=2.0)     # fast.py:138
-        speed = torch.where((steer.abs() < 0.1) & (r[:, 0] > 0.5), torch.full_like(slow, 7.0), slow)  # fast.py:135-136
-        self.raised = raised
-        return speed, steer
+    SPEED_DIVISOR = math.pi          # fast.py:138
+    BOOST_MAX_STEER = 0.1            # fast.py:135
+    SPEED_CAP = 2.0                  # fast.py:138

@@ -12,6 +12,7 @@ Mirrors what `Mujoco.physics_thread` touches every tick (ft_grandprix/custom.py:
     self.winners                                      fleet.lap[:, rank] / fleet.winners[world]
     mujoco.mj_step(model, data)                       fleet.step()
     driver.process_lidar(ranges)                      fleet.drive() (device) / fleet.drive_host()
+    the drivers' constants (nidc.py:5-10, fast.py:4-9) fleet.set_driver_params(rows): one row per car (DRV fields)
     reload() after every car has finished             Fleet(reload_finished=True): inside fleet.tick(), per world,
                                                       race results summed in fleet.race_tally (RACE_FIELDS)
 
@@ -26,16 +27,27 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import (DRIVER_FAST, DRIVER_LOBOTOMY, DRIVER_NIDC, LAP_FIELDS, MAX_LAPTIMES, NBEAMS, NQ, NU, NV, RACE_FIELDS)
+from ._lib import (DRIVER_FAST, DRIVER_LOBOTOMY, DRIVER_NIDC, DRV_FIELDS, LAP_FIELDS, MAX_LAPTIMES, NBEAMS, NQ, NU, NV,
+                   RACE_FIELDS)
+from .drivers import BatchedFastDriver, BatchedNidcDriver
 from .track import Geometry, Track
 from .vehicle import VehicleStateSnapshot
 
 TIMESTEP = 0.004                      # template/mushr.em.xml:30
 LAP = {name: k for k, name in enumerate(LAP_FIELDS)}
 RACE = {name: k for k, name in enumerate(RACE_FIELDS)}
+DRV = {name: k for k, name in enumerate(DRV_FIELDS)}
 DRIVER_KINDS = {"nidc": DRIVER_NIDC, "fast": DRIVER_FAST, "lobotomy": DRIVER_LOBOTOMY,
                 "ft_grandprix.nidc": DRIVER_NIDC, "ft_grandprix.fast": DRIVER_FAST,
                 "ft_grandprix.lobotomy": DRIVER_LOBOTOMY}
+
+def default_driver_params(kind):
+    """The reference parameter row (DRV fields, include/ftgp.h FTGP_DRV_*) of a bundled driver: 'nidc' or 'fast' (or
+    DRIVER_NIDC / DRIVER_FAST), as a float64 numpy array [10]."""
+    k = DRIVER_KINDS[kind] if isinstance(kind, str) else int(kind)
+    if k not in (DRIVER_NIDC, DRIVER_FAST):
+        raise ValueError("only the nidc and fast drivers have a parameter row")
+    return np.array((BatchedNidcDriver if k == DRIVER_NIDC else BatchedFastDriver).default_row(), dtype=np.float64)
 
 def _ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else None
@@ -79,6 +91,8 @@ class Fleet:
         self.status = torch.zeros(n, dtype=torch.int32, device=dev)
         self.track_id = None if track_id is None else torch.as_tensor(track_id, dtype=torch.int32).to(dev).contiguous()
         self.driver_kind = None
+        self.driver_params = None            # [ncars, len(DRV)] float64 rows (set_driver_params), None = reference constants
+        self._driver_params = None           # the rows' storage, allocated once (the tick's graph key holds its address)
         self.steps = 0
         if self.reload_finished:
             self.race_tally = torch.zeros(n, len(RACE_FIELDS), dtype=torch.int32, device=dev)
@@ -124,6 +138,28 @@ class Fleet:
         """Per-car built-in driver: names ('nidc', 'fast', 'lobotomy') or FTGP_DRIVER_* ints."""
         k = [DRIVER_KINDS[x] if isinstance(x, str) else int(x) for x in kinds]
         self.driver_kind = torch.tensor(k, dtype=torch.int32, device=self.device)
+
+    def set_driver_params(self, rows):
+        """Per-car constants of the device drivers: rows [ncars, len(DRV)] (or one row [len(DRV)] for every car), float64,
+        fields DRV (default_driver_params(kind) gives the reference rows).  With rows, a car's row alone decides its
+        disparity extender and speed law; driver kinds then only matter as 'lobotomy', and finished cars are still
+        lobotomised.  None returns to the reference constants of each car's kind.  The rows are copied into
+        fleet.driver_params in stream order (ticks already issued read the old rows); that tensor keeps its address, so
+        a graph-replayed tick reads new rows without a recapture, and writing into it in place on fleet.stream works
+        as well."""
+        if rows is None:
+            self.driver_params = None
+            return
+        rows = torch.as_tensor(rows, dtype=torch.float64, device=self.device)
+        if rows.shape not in ((len(DRV),), (self.ncars, len(DRV))):
+            raise ValueError(f"rows must be [ncars, {len(DRV)}] or [{len(DRV)}]")
+        if self._driver_params is None:
+            self._driver_params = torch.empty(self.ncars, len(DRV), dtype=torch.float64, device=self.device)
+        self.stream.wait_stream(torch.cuda.current_stream(self.device))
+        with torch.cuda.stream(self.stream):
+            self._driver_params.copy_(rows.expand(self.ncars, -1))
+        rows.record_stream(self.stream)
+        self.driver_params = self._driver_params
 
     def _grid_offsets(self):
         """VehicleState(offset=(i+5)*2) of grid slot i (custom.py:96-118)."""
@@ -233,8 +269,9 @@ class Fleet:
             with torch.cuda.stream(self.stream):
                 prev = self.ctrl.clone()
         if self.always_invoke_driver or not self.manual_control:
-            _lib.check(self.lib.ftgp_drivers(_ptr(self.ranges), _ptr(self.driver_kind), self.default_driver,
-                                             _ptr(self.lap), _ptr(self.ctrl), self.ncars, self._s), "ftgp_drivers")
+            _lib.check(self.lib.ftgp_drivers_params(_ptr(self.ranges), _ptr(self.driver_kind), self.default_driver,
+                                                    _ptr(self.driver_params), _ptr(self.lap), _ptr(self.ctrl), self.ncars,
+                                                    self._s), "ftgp_drivers_params")
         else:
             with torch.cuda.stream(self.stream):
                 self.ctrl.zero_()
@@ -256,7 +293,8 @@ class Fleet:
     def drive_host(self, drivers):
         """Slow path for unmodified reference-style drivers (SURVEY §8 B1): one Python object per car
         with process_lidar(ranges) or process_lidar(ranges, state); exceptions are printed and leave
-        that car's ctrl unchanged (custom.py:1403-1411)."""
+        that car's ctrl unchanged (custom.py:1403-1411).  fleet.driver_params is ignored: host drivers carry their
+        own constants."""
         import inspect
         self.sync()
         ranges = self.ranges.cpu().numpy().astype(np.float64)
@@ -340,11 +378,9 @@ class Fleet:
                 self.lap_update(); self.drive(); self.lidar(); self.step(1)
             return
         a = self.tick_args()
-        if self.reload_finished:
-            r = self.reload_args()
-            _lib.check(self.lib.ftgp_tick_reload(C.byref(a), C.byref(r), int(nticks), self._s), "ftgp_tick_reload")
-        else:
-            _lib.check(self.lib.ftgp_tick(C.byref(a), int(nticks), self._s), "ftgp_tick")
+        r = C.byref(self.reload_args()) if self.reload_finished else None
+        _lib.check(self.lib.ftgp_tick_params(C.byref(a), r, _ptr(self.driver_params), int(nticks), self._s),
+                   "ftgp_tick_params")
         self.steps += int(nticks)
 
     def tick_readback(self, ranges_host, lap_host, cars=None):
@@ -445,10 +481,15 @@ class Fleet:
         return keys
 
     def state_dict(self):
+        """The fleet's arrays on the host, with driver_params when rows are set."""
         self.sync()
-        return {k: getattr(self, k).cpu() for k in self._state_keys()} | {"steps": self.steps}
+        sd = {k: getattr(self, k).cpu() for k in self._state_keys()} | {"steps": self.steps}
+        if self.driver_params is not None:
+            sd["driver_params"] = self.driver_params.cpu()
+        return sd
 
     def load_state_dict(self, sd):
         for k in self._state_keys():
             getattr(self, k).copy_(sd[k])
+        self.set_driver_params(sd.get("driver_params"))
         self.steps = int(sd["steps"])

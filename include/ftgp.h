@@ -150,6 +150,43 @@ int ftgp_release_scratch(void* stream);
 int ftgp_drivers(const float* ranges, const int32_t* kind, int default_kind, const int32_t* lap,
                  double* ctrl, int64_t ncars, void* stream);
 
+/* Per-car driver parameters: the constants a competitor edits to tune the bundled disparity extender, as one fp64 row
+ * per car, params[ncars][FTGP_DRV_FIELDS].  One formula covers both bundled drivers (nidc.py:12-131, fast.py:12-139):
+ *   disparity at i >= 1 of proc = ranges[11:79]:  |proc[i] - proc[i-1]| > DIFFERENCE_THRESHOLD
+ *   cover width:        (CAR_WIDTH / 2) * (1 + SAFETY_PERCENTAGE / 100)                         nidc.py:93
+ *   covered beams:      ceil(2 * atan(width / (2 * dist)) / (2 pi / 90))                        nidc.py:57-58
+ *   steering st:        the chosen beam's angle clipped to [-MAX_STEER, MAX_STEER]             nidc.py:112-113
+ *   speed:              BOOST_SPEED                      if |st| < BOOST_MAX_STEER and ranges[0] > BOOST_MIN_REAR_RANGE
+ *                       s < SPEED_CAP ? s : SPEED_CAP    otherwise, s = SPEED * 5 * (1 - |st| / SPEED_DIVISOR)
+ *                                                                                               nidc.py:130, fast.py:135-138
+ * The reference instances (the rows used when params is NULL):
+ *   field                  nidc                               fast
+ *   CAR_WIDTH              0.12                               0.06                  nidc.py:5, fast.py:4
+ *   SAFETY_PERCENTAGE      300                                300                   nidc.py:10
+ *   DIFFERENCE_THRESHOLD   0.6                                0.6                   nidc.py:7
+ *   SPEED                  0.5                                0.5                   nidc.py:8
+ *   SPEED_DIVISOR          1.57 * 2                           3.141592653589793     nidc.py:130, fast.py:138
+ *   MAX_STEER              90.0 * (3.141592653589793 / 180.0) the same              nidc.py:113 (np.radians(90))
+ *   BOOST_SPEED            7                                  7                     fast.py:136
+ *   BOOST_MAX_STEER        0 (|st| < 0 never holds)           0.1                   fast.py:135
+ *   BOOST_MIN_REAR_RANGE   0.5                                0.5                   fast.py:135 (ranges[0]: the rear beam)
+ *   SPEED_CAP              +inf                               2                     fast.py:138
+ * The beam window (68 beams from index 11) is fixed.  Rows are not validated: an out-of-range row does exactly what the
+ * numpy formula does.  A NaN width (or inf width at inf range) raises at the first disparity and leaves ctrl unchanged,
+ * as custom.py:1409-1411 does; a zero or negative width covers nothing; a negative threshold makes every index whose
+ * difference is not NaN a disparity, an infinite or NaN one none; atan is bounded, so a disparity covers at most 45
+ * beams whatever the width; a NaN speed law gives SPEED_CAP; a NaN MAX_STEER clips nothing. */
+enum {
+    FTGP_DRV_CAR_WIDTH = 0, FTGP_DRV_SAFETY_PERCENTAGE, FTGP_DRV_DIFFERENCE_THRESHOLD, FTGP_DRV_SPEED,
+    FTGP_DRV_SPEED_DIVISOR, FTGP_DRV_MAX_STEER, FTGP_DRV_BOOST_SPEED, FTGP_DRV_BOOST_MAX_STEER,
+    FTGP_DRV_BOOST_MIN_REAR_RANGE, FTGP_DRV_SPEED_CAP, FTGP_DRV_FIELDS
+};
+/* ftgp_drivers with per-car rows: params = device double[ncars][FTGP_DRV_FIELDS] or NULL (= the reference row of each
+ * car's kind; ftgp_drivers is this call with NULL).  With rows, a car's row alone decides its driver: kind matters only
+ * as FTGP_DRIVER_LOBOTOMY, and finished cars still run the lobotomy driver. */
+int ftgp_drivers_params(const float* ranges, const int32_t* kind, int default_kind, const double* params,
+                        const int32_t* lap, double* ctrl, int64_t ncars, void* stream);
+
 /* ------------------------------------------------------------------ lap logic */
 /* Replaces custom.py:1340-1372.  lap: device int32[ncars][FTGP_LAP_FIELDS] (see enum),
  * times: device int32[ncars][FTGP_MAX_LAPTIMES] lap durations in steps (x 0.004 s),
@@ -220,6 +257,11 @@ typedef struct {
 int ftgp_reload(const ftgp_tick_args* a, const ftgp_reload_args* r, void* stream);
 /* ftgp_tick with the reload at the head of every tick (graph-replayed like ftgp_tick); r == NULL is exactly ftgp_tick. */
 int ftgp_tick_reload(const ftgp_tick_args* a, const ftgp_reload_args* r, int nticks, void* stream);
+/* ftgp_tick_reload whose drivers read per-car rows (driver_params: device double[ncars][FTGP_DRV_FIELDS] or NULL, see
+ * ftgp_drivers_params); ftgp_tick_reload is this call with NULL.  The rows are read by every tick, graph-replayed ones
+ * included, so rewriting them in place, in stream order, takes effect on the next tick. */
+int ftgp_tick_params(const ftgp_tick_args* a, const ftgp_reload_args* r, const double* driver_params, int nticks,
+                     void* stream);
 /* enable != 0 (default): small fleets replay the captured tick; 0: every tick is issued launch by launch.
  * Returns the previous setting (for A/B timing in the bench). */
 int ftgp_tick_use_graphs(int enable);
