@@ -5,6 +5,7 @@ Everything numeric lives in libftgp.so (csrc/*.cu, C ABI in include/ftgp.h).  Im
 package loads that library and fails loudly if it has not been built."""
 from . import _lib
 from .drivers import BatchedFastDriver, BatchedLobotomyDriver, BatchedNidcDriver, LobotomyDriver
+from .policy import PolicyNet, policy_inputs
 from .track import Geometry, Track, centreline
 from .vehicle import VehicleStateSnapshot
 

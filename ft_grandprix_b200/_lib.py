@@ -15,7 +15,7 @@ LAP_FIELDS = ("offset", "completion", "laps", "start", "good_start", "finished",
               "off_track", "rank", "delta", "offtrack_ticks", "contact_ticks")
 RACE_FIELDS = ("races", "finished", "wins", "rank_sum", "laps_sum", "time_sum", "best_lap", "offtrack_ticks",
                "contact_ticks")
-DRIVER_NIDC, DRIVER_FAST, DRIVER_LOBOTOMY = 0, 1, 2
+DRIVER_NIDC, DRIVER_FAST, DRIVER_LOBOTOMY, DRIVER_POLICY = 0, 1, 2, 3
 DRV_FIELDS = ("car_width", "safety_percentage", "difference_threshold", "speed", "speed_divisor", "max_steer",
               "boost_speed", "boost_max_steer", "boost_min_rear_range", "speed_cap")
 OPT_NAIVE_FLATTEN, OPT_BUBBLE_WRAP = 1, 2
@@ -35,6 +35,9 @@ class TickArgs(C.Structure):
 class ReloadArgs(C.Structure):
     _fields_ = [("start_xy", C.c_void_p), ("start_yaw", C.c_void_p), ("start_offset", C.c_void_p),
                 ("race_start", C.c_void_p), ("tally", C.c_void_p), ("race_ticks", C.c_int32), ("reserved", C.c_int32)]
+
+class PolicyArgs(C.Structure):
+    _fields_ = [("weights", C.c_void_p), ("policy_id", C.c_void_p), ("npolicies", C.c_int32), ("reserved", C.c_int32)]
 
 _vp, _i, _i64, _d = C.c_void_p, C.c_int, C.c_int64, C.c_double
 # name -> (restype, argtypes); mirrors include/ftgp.h one to one
@@ -68,6 +71,8 @@ SIGNATURES = {
     "ftgp_reload": (_i, [C.POINTER(TickArgs), C.POINTER(ReloadArgs), _vp]),
     "ftgp_tick_reload": (_i, [C.POINTER(TickArgs), C.POINTER(ReloadArgs), _i, _vp]),
     "ftgp_tick_params": (_i, [C.POINTER(TickArgs), C.POINTER(ReloadArgs), _vp, _i, _vp]),
+    "ftgp_drivers_policy": (_i, [_vp, _vp, _i, _vp, C.POINTER(PolicyArgs), _vp, _vp, _vp, _vp, _i64, _vp]),
+    "ftgp_tick_policy": (_i, [C.POINTER(TickArgs), C.POINTER(ReloadArgs), _vp, C.POINTER(PolicyArgs), _i, _vp]),
 }
 
 _lib = None

@@ -18,6 +18,19 @@ void count_launch(int n = 1);
         if (!ftgp::cuda_ok((call), #call)) return FTGP_ERR_CUDA; \
     } while (0)
 
+// ---- policy bank (policy.cu) ----------------------------------------------
+// checked before any CUDA call: a bank needs weights and at least one policy; FTGP_DRIVER_POLICY as the default needs a bank
+inline bool bad_policy_args(const ftgp_policy_args* p, int default_kind) {
+    if (!p) return default_kind == FTGP_DRIVER_POLICY;
+    return !p->weights || p->npolicies < 1;
+}
+// the POLICY cars of the fleet, grouped by policy id, then evaluated (after drivers_kernel, which skips them)
+int launch_policy(const ftgp_policy_args* p, const float* ranges, const int32_t* kind, int default_kind, const double* qpos,
+                  const double* qvel, const int32_t* lap, double* ctrl, int64_t ncars, cudaStream_t stream);
+// the per-stream scratch of the grouping (step.cu keeps it with the step's, so captured ticks see it re-allocated):
+// int32 hist[npolicies], cursor[npolicies], total[1], list[ncars]
+int policy_scratch(int64_t ncars, int npolicies, cudaStream_t stream, int32_t** buf);
+
 // ---- device geometry blob -------------------------------------------------
 // One blob per ftgp_geom, replicated on a GPU and staged into shared memory by
 // the lidar kernel.  All offsets are in 32-bit words from the start of the blob.

@@ -167,7 +167,7 @@ template <int F> __device__ __forceinline__ double drv(const double* __restrict_
 __global__ void __launch_bounds__(256)
 drivers_kernel(const float* __restrict__ ranges, const int32_t* __restrict__ kind, int default_kind,
                const double* __restrict__ params, const int32_t* __restrict__ lap, double* __restrict__ ctrl, int64_t ncars,
-               int32_t* __restrict__ steps_dev) {
+               int32_t* __restrict__ steps_dev, bool bank) {
     const int lane = threadIdx.x & 31;
     const int64_t car = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     // graph-replayed tick: the lap kernel (earlier on this stream) has read the tick counter; nothing else reads it this tick
@@ -175,6 +175,10 @@ drivers_kernel(const float* __restrict__ ranges, const int32_t* __restrict__ kin
     if (car >= ncars) return;
     int k = kind ? kind[car] : default_kind;
     if (lap && lap[car * FTGP_LAP_FIELDS + FTGP_LAP_FINISHED]) k = FTGP_DRIVER_LOBOTOMY;   // shadow(): custom.py:1437
+    if (k == FTGP_DRIVER_POLICY) {                  // policy_kernel (policy.cu) drives it; without a bank it is inert
+        if (bank) return;
+        k = FTGP_DRIVER_LOBOTOMY;
+    }
     double* out = ctrl + 2 * car;
     if (k == FTGP_DRIVER_LOBOTOMY) { if (lane == 0) { out[0] = 0.0; out[1] = 0.0; } return; }
     const double* prow = params ? params + car * FTGP_DRV_FIELDS : nullptr;
@@ -321,10 +325,10 @@ __global__ void lap_kernel(const uint32_t* __restrict__ blob, const double* __re
 }
 
 int launch_drivers(const float* ranges, const int32_t* kind, int default_kind, const double* params, const int32_t* lap,
-                   double* ctrl, int64_t ncars, cudaStream_t stream, int32_t* steps_dev) {
+                   double* ctrl, int64_t ncars, cudaStream_t stream, int32_t* steps_dev, bool bank) {
     const int threads = 256;
     int64_t blocks = (ncars * 32 + threads - 1) / threads;
-    drivers_kernel<<<(unsigned)blocks, threads, 0, stream>>>(ranges, kind, default_kind, params, lap, ctrl, ncars, steps_dev);
+    drivers_kernel<<<(unsigned)blocks, threads, 0, stream>>>(ranges, kind, default_kind, params, lap, ctrl, ncars, steps_dev, bank);
     count_launch();
     FTGP_CUDA(cudaGetLastError());
     return FTGP_OK;
@@ -361,11 +365,20 @@ extern "C" int ftgp_naive_flatten(double* qpos, int64_t qpos_stride, int64_t nca
     return launch_flatten(qpos, qpos_stride, ncars, (cudaStream_t)stream);
 }
 
+extern "C" int ftgp_drivers_policy(const float* ranges, const int32_t* kind, int default_kind, const double* params,
+                                   const ftgp_policy_args* policy, const double* qpos, const double* qvel, const int32_t* lap,
+                                   double* ctrl, int64_t ncars, void* stream) {
+    if (!ranges || !ctrl || ncars < 0 || default_kind < 0 || default_kind > FTGP_DRIVER_POLICY) { set_error("ftgp_drivers: bad argument"); return FTGP_ERR_ARG; }
+    if (bad_policy_args(policy, default_kind) || (policy && (!qpos || !qvel))) { set_error("ftgp_drivers: bad policy argument"); return FTGP_ERR_ARG; }
+    if (ncars == 0) return FTGP_OK;
+    int rc = launch_drivers(ranges, kind, default_kind, params, lap, ctrl, ncars, (cudaStream_t)stream, nullptr, policy != nullptr);
+    if (!rc && policy) rc = launch_policy(policy, ranges, kind, default_kind, qpos, qvel, lap, ctrl, ncars, (cudaStream_t)stream);
+    return rc;
+}
+
 extern "C" int ftgp_drivers_params(const float* ranges, const int32_t* kind, int default_kind, const double* params,
                                    const int32_t* lap, double* ctrl, int64_t ncars, void* stream) {
-    if (!ranges || !ctrl || ncars < 0 || default_kind < 0 || default_kind > 2) { set_error("ftgp_drivers: bad argument"); return FTGP_ERR_ARG; }
-    if (ncars == 0) return FTGP_OK;
-    return launch_drivers(ranges, kind, default_kind, params, lap, ctrl, ncars, (cudaStream_t)stream, nullptr);
+    return ftgp_drivers_policy(ranges, kind, default_kind, params, nullptr, nullptr, nullptr, lap, ctrl, ncars, stream);
 }
 
 extern "C" int ftgp_drivers(const float* ranges, const int32_t* kind, int default_kind, const int32_t* lap,

@@ -159,6 +159,7 @@ struct StepScratch {
     int32_t* world_list = nullptr; uint8_t* world_flag = nullptr; int64_t world_cap = 0;                                // coupled worlds
     void* world_spill = nullptr;                                                                                         // workspaces of warps 1.. of world_step_kernel
     double* qpos_snap = nullptr; int64_t snap_cap = 0;      // fused tick: the poses the rangefinders read while the coupled worlds already move
+    int32_t* policy = nullptr; int64_t policy_cars = 0; int policy_banks = 0;   // policy.cu: the POLICY cars grouped by policy id
     bool world_inflight = false;                            // the coupled worlds of this step were started by launch_worlds_early
     cudaStream_t side = nullptr; cudaEvent_t ev_fork = nullptr, ev_join = nullptr;       // ... advanced beside the fast path
     cudaStream_t scan = nullptr; cudaEvent_t ev_scan_fork = nullptr, ev_scan_join = nullptr;    // fused tick: the rangefinders beside the step
@@ -182,6 +183,7 @@ struct StepScratch {
         if (world_flag) cudaFree(world_flag);
         if (world_spill) cudaFree(world_spill);
         if (qpos_snap) cudaFree(qpos_snap);
+        if (policy) cudaFree(policy);
         cudaSetDevice(cur);
         const uint64_t gen = generation + 1;
         *this = StepScratch();
@@ -458,7 +460,22 @@ int launch_lidar(const ftgp_geom* g, const double* qpos, int64_t stride, const i
                  const uint8_t* visible, const int32_t* lap, int64_t ncars, int cpw, float* ranges, float* min_range,
                  cudaStream_t stream);
 int launch_drivers(const float* ranges, const int32_t* kind, int default_kind, const double* params, const int32_t* lap,
-                   double* ctrl, int64_t ncars, cudaStream_t stream, int32_t* steps_dev);
+                   double* ctrl, int64_t ncars, cudaStream_t stream, int32_t* steps_dev, bool bank);
+
+int policy_scratch(int64_t ncars, int npolicies, cudaStream_t stream, int32_t** buf) {
+    int dev = 0;
+    FTGP_CUDA(cudaGetDevice(&dev));
+    std::lock_guard<std::mutex> lock(g_step_mutex);
+    StepScratch* o = step_scratch(dev, stream);
+    if (o->policy_cars < ncars || o->policy_banks < npolicies) {
+        if (o->policy) cudaFree(o->policy);
+        o->policy = nullptr; o->policy_cars = 0; o->policy_banks = 0; o->generation++;
+        FTGP_CUDA(cudaMalloc(&o->policy, (size_t)(2 * (int64_t)npolicies + 1 + ncars) * sizeof(int32_t)));
+        o->policy_cars = ncars; o->policy_banks = npolicies;
+    }
+    *buf = o->policy;
+    return FTGP_OK;
+}
 int launch_lap(const ftgp_geom* g, const double* qpos, int64_t stride, const int32_t* track_id, int32_t* lap,
                int32_t* times, int32_t* winners, const int32_t* status, int64_t ncars, int cpw, int32_t steps,
                int32_t lap_target, cudaStream_t stream, const int32_t* steps_dev);
@@ -499,9 +516,10 @@ static int overlap_fork(double* qpos, int64_t ncars, bool copy, cudaStream_t str
 }
 
 // ---- one tick = custom.py:1337-1426 for the whole fleet, in the reference's order; r != NULL: the worlds whose race is
-// over are reloaded first (custom.py:1089-1128); dp != NULL: the drivers read the per-car rows (ftgp_drivers_params)
-static int issue_tick(const ftgp_tick_args* a, const ftgp_reload_args* r, const double* dp, int32_t steps, int32_t* steps_dev,
-                      cudaStream_t s) {
+// over are reloaded first (custom.py:1089-1128); dp != NULL: the drivers read the per-car rows (ftgp_drivers_params);
+// pa != NULL: the POLICY cars run the bank (ftgp_drivers_policy), right after the other drivers
+static int issue_tick(const ftgp_tick_args* a, const ftgp_reload_args* r, const double* dp, const ftgp_policy_args* pa, int32_t steps,
+                      int32_t* steps_dev, cudaStream_t s) {
     int rc;
     if (r && (rc = launch_reload(a, r, steps, s, steps_dev))) return rc;
     // custom.py:1338-1339 option naive_flatten
@@ -510,7 +528,8 @@ static int issue_tick(const ftgp_tick_args* a, const ftgp_reload_args* r, const 
     if ((rc = launch_lap(a->geom, a->qpos, FTGP_NQ, a->track_id, a->lap, a->times, a->winners, a->status, a->ncars,
                          a->cars_per_world, steps, a->lap_target, s, steps_dev))) return rc;
     // custom.py:1395-1423 driver on the ranges of the previous mj_step, control write
-    if ((rc = launch_drivers(a->ranges, a->driver_kind, a->default_driver, dp, a->lap, a->ctrl, a->ncars, s, steps_dev))) return rc;
+    if ((rc = launch_drivers(a->ranges, a->driver_kind, a->default_driver, dp, a->lap, a->ctrl, a->ncars, s, steps_dev, pa != nullptr))) return rc;
+    if (pa && (rc = launch_policy(pa, a->ranges, a->driver_kind, a->default_driver, a->qpos, a->qvel, a->lap, a->ctrl, a->ncars, s))) return rc;
     // custom.py:1425 mj_step: rangefinders are evaluated from the pre-step pose, then the state advances.  The rangefinder
     // kernel scans a copy of the poses on a stream of its own beside the step; in worlds of several cars the coupled worlds'
     // solver starts here as well, on a third stream (launch_worlds_early takes the copy in that case).
@@ -533,6 +552,7 @@ constexpr int64_t GRAPH_MAX_CARS = 16384;
 static std::atomic<int> g_use_graphs{1};
 struct TickGraph {
     ftgp_tick_args key{}; bool reload = false; ftgp_reload_args rkey{}; const double* params = nullptr;
+    bool policy = false; ftgp_policy_args pkey{};
     cudaStream_t stream = nullptr; int dev = -1;
     cudaGraphExec_t exec = nullptr; int32_t* steps_dev = nullptr; int32_t shadow = INT32_MIN;
     uint64_t scratch_gen = 0; int launches_per_tick = 0; bool seen = false; uint64_t used = 0;
@@ -559,6 +579,11 @@ static bool same_reload(const TickGraph& g, const ftgp_reload_args* r) {
     return g.reload && x.start_xy == r->start_xy && x.start_yaw == r->start_yaw && x.start_offset == r->start_offset &&
            x.race_start == r->race_start && x.tally == r->tally && x.race_ticks == r->race_ticks;
 }
+static bool same_policy(const TickGraph& g, const ftgp_policy_args* p) {
+    if (!p) return !g.policy;
+    const ftgp_policy_args& x = g.pkey;
+    return g.policy && x.weights == p->weights && x.policy_id == p->policy_id && x.npolicies == p->npolicies;
+}
 static void drop_graph(TickGraph& g) {
     if (g.exec) cudaGraphExecDestroy(g.exec);
     if (g.steps_dev) cudaFree(g.steps_dev);
@@ -566,8 +591,8 @@ static void drop_graph(TickGraph& g) {
 }
 
 // returns FTGP_OK and sets *done = number of ticks issued through the graph (0: caller runs them eagerly)
-static int graph_ticks(const ftgp_tick_args* a, const ftgp_reload_args* r, const double* dp, int nticks, cudaStream_t s,
-                       int* done) {
+static int graph_ticks(const ftgp_tick_args* a, const ftgp_reload_args* r, const double* dp, const ftgp_policy_args* pa, int nticks,
+                       cudaStream_t s, int* done) {
     *done = 0;
     int dev = 0;
     FTGP_CUDA(cudaGetDevice(&dev));
@@ -575,7 +600,7 @@ static int graph_ticks(const ftgp_tick_args* a, const ftgp_reload_args* r, const
     TickGraph* e = nullptr; TickGraph* lru = &g_graphs[0];
     for (auto& g : g_graphs) {
         if (g.seen && g.dev == dev && g.stream == s && same_key(g.key, *a) && same_reload(g, r) &&
-            g.params == dp) { e = &g; break; }
+            g.params == dp && same_policy(g, pa)) { e = &g; break; }
         if (g.used < lru->used) lru = &g;
     }
     int32_t steps = a->steps;
@@ -585,8 +610,10 @@ static int graph_ticks(const ftgp_tick_args* a, const ftgp_reload_args* r, const
         lru->reload = r != nullptr;
         if (r) lru->rkey = *r;
         lru->params = dp;
+        lru->policy = pa != nullptr;
+        if (pa) lru->pkey = *pa;
         e = lru;
-        const int rc = issue_tick(a, r, dp, steps, nullptr, s);
+        const int rc = issue_tick(a, r, dp, pa, steps, nullptr, s);
         if (rc) return rc;
         steps++; nticks--; *done = 1;
         if (nticks == 0) { e->used = ++g_graph_clock; return FTGP_OK; }
@@ -599,7 +626,7 @@ static int graph_ticks(const ftgp_tick_args* a, const ftgp_reload_args* r, const
         const int64_t l0 = ftgp_launch_count();
         cudaGraph_t graph = nullptr;
         FTGP_CUDA(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-        const int rc = issue_tick(a, r, dp, 0, e->steps_dev, s);
+        const int rc = issue_tick(a, r, dp, pa, 0, e->steps_dev, s);
         const cudaError_t ce = cudaStreamEndCapture(s, &graph);
         if (rc || ce != cudaSuccess || !graph) {                 // capture refused (e.g. scratch had to grow): stay eager
             if (graph) cudaGraphDestroy(graph);
@@ -654,20 +681,29 @@ static bool bad_reload_args(const ftgp_reload_args* r) {
            (r->tally && !r->race_start) || (r->race_ticks > 0 && !r->race_start);
 }
 
-extern "C" int ftgp_tick_params(const ftgp_tick_args* a, const ftgp_reload_args* r, const double* driver_params, int nticks,
-                                void* stream) {
+extern "C" int ftgp_tick_policy(const ftgp_tick_args* a, const ftgp_reload_args* r, const double* driver_params,
+                                const ftgp_policy_args* policy, int nticks, void* stream) {
     if (bad_tick_args(a) || nticks < 0) { set_error("ftgp_tick: bad argument"); return FTGP_ERR_ARG; }
     if (r && bad_reload_args(r)) { set_error("ftgp_tick_reload: bad reload argument"); return FTGP_ERR_ARG; }
+    if (bad_policy_args(policy, a->default_driver) ||
+        (policy && (a->default_driver < 0 || a->default_driver > FTGP_DRIVER_POLICY))) {
+        set_error("ftgp_tick_policy: bad policy argument"); return FTGP_ERR_ARG;
+    }
     if (a->ncars == 0 || nticks == 0) return FTGP_OK;
     FTGP_CUDA(cudaSetDevice(a->geom->device));
     cudaStream_t s = (cudaStream_t)stream;
     int t0 = 0, rc;
     if (a->ncars <= GRAPH_MAX_CARS && s != nullptr && g_use_graphs.load()) {           // (the legacy default stream cannot be captured)
-        if ((rc = graph_ticks(a, r, driver_params, nticks, s, &t0))) return rc;
+        if ((rc = graph_ticks(a, r, driver_params, policy, nticks, s, &t0))) return rc;
     }
     for (int t = t0; t < nticks; t++)
-        if ((rc = issue_tick(a, r, driver_params, a->steps + t, nullptr, s))) return rc;
+        if ((rc = issue_tick(a, r, driver_params, policy, a->steps + t, nullptr, s))) return rc;
     return FTGP_OK;
+}
+
+extern "C" int ftgp_tick_params(const ftgp_tick_args* a, const ftgp_reload_args* r, const double* driver_params, int nticks,
+                                void* stream) {
+    return ftgp_tick_policy(a, r, driver_params, nullptr, nticks, stream);
 }
 
 extern "C" int ftgp_tick_reload(const ftgp_tick_args* a, const ftgp_reload_args* r, int nticks, void* stream) {

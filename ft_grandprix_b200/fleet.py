@@ -15,6 +15,8 @@ Mirrors what `Mujoco.physics_thread` touches every tick (ft_grandprix/custom.py:
     the drivers' constants (nidc.py:5-10, fast.py:4-9) fleet.set_driver_params(rows): one row per car (DRV fields)
     reload() after every car has finished             Fleet(reload_finished=True): inside fleet.tick(), per world,
                                                       race results summed in fleet.race_tally (RACE_FIELDS)
+    a driver of any shape (a learned one)             kind "policy": one MLP of a bank per car, fleet.set_policies(bank,
+                                                      policy_id); the torch twin is ft_grandprix_b200.policy.PolicyNet
 
 All arithmetic runs in libftgp.so (hand-written sm_100a CUDA behind include/ftgp.h); torch only
 owns the device memory and the stream.  There is no CPU fallback: constructing a Fleet without a
@@ -27,9 +29,10 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import (DRIVER_FAST, DRIVER_LOBOTOMY, DRIVER_NIDC, DRV_FIELDS, LAP_FIELDS, MAX_LAPTIMES, NBEAMS, NQ, NU, NV,
-                   RACE_FIELDS)
+from ._lib import (DRIVER_FAST, DRIVER_LOBOTOMY, DRIVER_NIDC, DRIVER_POLICY, DRV_FIELDS, LAP_FIELDS, MAX_LAPTIMES, NBEAMS,
+                   NQ, NU, NV, RACE_FIELDS)
 from .drivers import BatchedFastDriver, BatchedNidcDriver
+from .policy import POLICY_FLOATS
 from .track import Geometry, Track
 from .vehicle import VehicleStateSnapshot
 
@@ -37,7 +40,7 @@ TIMESTEP = 0.004                      # template/mushr.em.xml:30
 LAP = {name: k for k, name in enumerate(LAP_FIELDS)}
 RACE = {name: k for k, name in enumerate(RACE_FIELDS)}
 DRV = {name: k for k, name in enumerate(DRV_FIELDS)}
-DRIVER_KINDS = {"nidc": DRIVER_NIDC, "fast": DRIVER_FAST, "lobotomy": DRIVER_LOBOTOMY,
+DRIVER_KINDS = {"nidc": DRIVER_NIDC, "fast": DRIVER_FAST, "lobotomy": DRIVER_LOBOTOMY, "policy": DRIVER_POLICY,
                 "ft_grandprix.nidc": DRIVER_NIDC, "ft_grandprix.fast": DRIVER_FAST,
                 "ft_grandprix.lobotomy": DRIVER_LOBOTOMY}
 
@@ -93,6 +96,9 @@ class Fleet:
         self.driver_kind = None
         self.driver_params = None            # [ncars, len(DRV)] float64 rows (set_driver_params), None = reference constants
         self._driver_params = None           # the rows' storage, allocated once (the tick's graph key holds its address)
+        self.policy_bank = None              # [P, POLICY_FLOATS] float32 (set_policies), None = no bank
+        self.policy_id = None                # [ncars] int32, or None = every POLICY car on policy 0
+        self._policy_id = None               # the ids' storage, allocated once
         self.steps = 0
         if self.reload_finished:
             self.race_tally = torch.zeros(n, len(RACE_FIELDS), dtype=torch.int32, device=dev)
@@ -135,7 +141,7 @@ class Fleet:
         self.stream.synchronize()
 
     def set_driver_kinds(self, kinds):
-        """Per-car built-in driver: names ('nidc', 'fast', 'lobotomy') or FTGP_DRIVER_* ints."""
+        """Per-car built-in driver: names ('nidc', 'fast', 'lobotomy', 'policy') or FTGP_DRIVER_* ints."""
         k = [DRIVER_KINDS[x] if isinstance(x, str) else int(x) for x in kinds]
         self.driver_kind = torch.tensor(k, dtype=torch.int32, device=self.device)
 
@@ -160,6 +166,50 @@ class Fleet:
             self._driver_params.copy_(rows.expand(self.ncars, -1))
         rows.record_stream(self.stream)
         self.driver_params = self._driver_params
+
+    def set_policies(self, bank, policy_id=None):
+        """The bank of neural-network drivers (ft_grandprix_b200.policy): bank [P, POLICY_FLOATS] float32 packed policies
+        (PolicyNet.pack()), policy_id [ncars] int32 (None: every car on policy 0).  Cars of kind 'policy' run policy
+        policy_id[car]; an id outside [0, P) drives (0, 0), finished cars are lobotomised, other kinds are unaffected.
+        None removes the bank (POLICY cars then drive (0, 0)).  The arrays are copied into fleet.policy_bank /
+        fleet.policy_id in stream order; those tensors keep their addresses while P stays the same, so a graph-replayed
+        tick reads a bank rewritten in place on fleet.stream without a recapture."""
+        if bank is None:
+            self.policy_bank = self.policy_id = None
+            return
+        bank = torch.as_tensor(bank, dtype=torch.float32, device=self.device)
+        if bank.dim() == 1:
+            bank = bank[None]
+        if bank.dim() != 2 or bank.shape[1] != POLICY_FLOATS or bank.shape[0] < 1:
+            raise ValueError(f"bank must be [P, {POLICY_FLOATS}] with P >= 1")
+        ids = None
+        if policy_id is not None:
+            ids = torch.as_tensor(policy_id, dtype=torch.int32, device=self.device)
+            if ids.shape != (self.ncars,):
+                raise ValueError("policy_id must be [ncars]")
+        if self.policy_bank is None or self.policy_bank.shape != bank.shape:
+            self.policy_bank = torch.empty_like(bank)
+        if ids is not None and self._policy_id is None:
+            self._policy_id = torch.empty(self.ncars, dtype=torch.int32, device=self.device)
+        self.stream.wait_stream(torch.cuda.current_stream(self.device))
+        with torch.cuda.stream(self.stream):
+            self.policy_bank.copy_(bank)
+            if ids is not None:
+                self._policy_id.copy_(ids)
+        for t in (bank, ids):
+            if t is not None:
+                t.record_stream(self.stream)
+        self.policy_id = None if ids is None else self._policy_id
+
+    def policy_args(self):
+        """ftgp_policy_args of the bank, or None without one."""
+        if self.policy_bank is None:
+            return None
+        p = _lib.PolicyArgs()
+        p.weights = self.policy_bank.data_ptr()
+        p.policy_id = None if self.policy_id is None else self.policy_id.data_ptr()
+        p.npolicies = self.policy_bank.shape[0]
+        return p
 
     def _grid_offsets(self):
         """VehicleState(offset=(i+5)*2) of grid slot i (custom.py:96-118)."""
@@ -269,9 +319,11 @@ class Fleet:
             with torch.cuda.stream(self.stream):
                 prev = self.ctrl.clone()
         if self.always_invoke_driver or not self.manual_control:
-            _lib.check(self.lib.ftgp_drivers_params(_ptr(self.ranges), _ptr(self.driver_kind), self.default_driver,
-                                                    _ptr(self.driver_params), _ptr(self.lap), _ptr(self.ctrl), self.ncars,
-                                                    self._s), "ftgp_drivers_params")
+            p = self.policy_args()
+            _lib.check(self.lib.ftgp_drivers_policy(_ptr(self.ranges), _ptr(self.driver_kind), self.default_driver,
+                                                    _ptr(self.driver_params), None if p is None else C.byref(p),
+                                                    _ptr(self.qpos), _ptr(self.qvel), _ptr(self.lap), _ptr(self.ctrl),
+                                                    self.ncars, self._s), "ftgp_drivers_policy")
         else:
             with torch.cuda.stream(self.stream):
                 self.ctrl.zero_()
@@ -294,7 +346,7 @@ class Fleet:
         """Slow path for unmodified reference-style drivers (SURVEY §8 B1): one Python object per car
         with process_lidar(ranges) or process_lidar(ranges, state); exceptions are printed and leave
         that car's ctrl unchanged (custom.py:1403-1411).  fleet.driver_params is ignored: host drivers carry their
-        own constants."""
+        own constants; so is the policy bank."""
         import inspect
         self.sync()
         ranges = self.ranges.cpu().numpy().astype(np.float64)
@@ -379,8 +431,9 @@ class Fleet:
             return
         a = self.tick_args()
         r = C.byref(self.reload_args()) if self.reload_finished else None
-        _lib.check(self.lib.ftgp_tick_params(C.byref(a), r, _ptr(self.driver_params), int(nticks), self._s),
-                   "ftgp_tick_params")
+        p = self.policy_args()
+        _lib.check(self.lib.ftgp_tick_policy(C.byref(a), r, _ptr(self.driver_params), None if p is None else C.byref(p),
+                                             int(nticks), self._s), "ftgp_tick_policy")
         self.steps += int(nticks)
 
     def tick_readback(self, ranges_host, lap_host, cars=None):
@@ -481,15 +534,20 @@ class Fleet:
         return keys
 
     def state_dict(self):
-        """The fleet's arrays on the host, with driver_params when rows are set."""
+        """The fleet's arrays on the host, with driver_params when rows are set and policy_bank / policy_id when a bank is."""
         self.sync()
         sd = {k: getattr(self, k).cpu() for k in self._state_keys()} | {"steps": self.steps}
         if self.driver_params is not None:
             sd["driver_params"] = self.driver_params.cpu()
+        if self.policy_bank is not None:
+            sd["policy_bank"] = self.policy_bank.cpu()
+            if self.policy_id is not None:
+                sd["policy_id"] = self.policy_id.cpu()
         return sd
 
     def load_state_dict(self, sd):
         for k in self._state_keys():
             getattr(self, k).copy_(sd[k])
         self.set_driver_params(sd.get("driver_params"))
+        self.set_policies(sd.get("policy_bank"), sd.get("policy_id"))
         self.steps = int(sd["steps"])

@@ -43,7 +43,7 @@ enum {
     FTGP_ERR_UNSUPPORTED = 4
 };
 
-enum { FTGP_DRIVER_NIDC = 0, FTGP_DRIVER_FAST = 1, FTGP_DRIVER_LOBOTOMY = 2 };
+enum { FTGP_DRIVER_NIDC = 0, FTGP_DRIVER_FAST = 1, FTGP_DRIVER_LOBOTOMY = 2, FTGP_DRIVER_POLICY = 3 };
 enum { FTGP_OPT_NAIVE_FLATTEN = 1, FTGP_OPT_BUBBLE_WRAP = 2 };   /* path-relevant options of custom.py:946-989 */
 
 const char* ftgp_last_error(void);
@@ -183,9 +183,53 @@ enum {
 };
 /* ftgp_drivers with per-car rows: params = device double[ncars][FTGP_DRV_FIELDS] or NULL (= the reference row of each
  * car's kind; ftgp_drivers is this call with NULL).  With rows, a car's row alone decides its driver: kind matters only
- * as FTGP_DRIVER_LOBOTOMY, and finished cars still run the lobotomy driver. */
+ * as FTGP_DRIVER_LOBOTOMY or FTGP_DRIVER_POLICY, and finished cars still run the lobotomy driver.
+ * ftgp_drivers_params is ftgp_drivers_policy (below) with no policy bank. */
 int ftgp_drivers_params(const float* ranges, const int32_t* kind, int default_kind, const double* params,
                         const int32_t* lap, double* ctrl, int64_t ncars, void* stream);
+
+/* Neural-network drivers: a car of kind FTGP_DRIVER_POLICY runs one policy of a bank, a small MLP of one fixed
+ * architecture, fp32.  Inputs x[96], computed per car at the driver's point of the tick (after the lap update, before
+ * the step; the ranges are the previous step's, as for the other kinds):
+ *   x[j], j = 0..89   r = ranges[j]; (r >= 0 && r < range_clip) ? r / range_clip : 1   (a miss, r >= clip and NaN give 1)
+ *   x[90], x[91]      forward and lateral speed in the yaw frame, yaw = atan2(2(wz + xy), 1 - 2(y^2 + z^2)) of qpos[3:7]
+ *                     (quaternion_to_euler, custom.py:62-76): fwd = vx cos yaw + vy sin yaw, lat = -vx sin yaw + vy cos yaw,
+ *                     (vx, vy) = qvel[0:2]; computed in fp64, rounded to fp32
+ *   x[92]             qvel[5]: the free joint's angular velocity about the chassis z axis
+ *   x[93], x[94]      the car's ctrl (speed, steering) at the head of the tick (zero after a reset or a reload)
+ *   x[95]             0 (padding)
+ * Network, hidden width 64, accurate tanhf:
+ *   h1 = tanh(b1 + W1^T x),  h2 = tanh(b2 + W2^T h1),  z = b3 + W3^T h2
+ *   speed = speed_scale * tanh(z0),  steering = steer_scale * tanh(z1)
+ * Every pre-activation is summed in input order, one fused multiply-add per input, starting from the bias, whatever
+ * other cars are evaluated with the car: a car's output does not depend on how cars are grouped.
+ * One policy = FTGP_POLICY_FLOATS floats (42,016 bytes; every block 16-byte aligned), weights input-major
+ * (W[i * width + j] multiplies input i into unit j: the transpose of torch.nn.Linear.weight):
+ *   FTGP_POLICY_SCALARS  range_clip, speed_scale, steer_scale, 0
+ *   FTGP_POLICY_W1       W1[96][64]        FTGP_POLICY_B1   b1[64]
+ *   FTGP_POLICY_W2       W2[64][64]        FTGP_POLICY_B2   b2[64]
+ *   FTGP_POLICY_W3       W3[64][2]         FTGP_POLICY_B3   b3[2], 2 floats of padding
+ * A POLICY car runs policy policy_id[car] (policy_id NULL: policy 0).  Finished cars run the lobotomy driver; an id
+ * outside [0, npolicies) writes (0, 0), as the reference's inert driver on an import failure (custom.py:1106-1109).  The
+ * output is written as computed.  Without a bank a POLICY car writes (0, 0). */
+enum {
+    FTGP_POLICY_NIN = 96, FTGP_POLICY_HIDDEN = 64, FTGP_POLICY_NOUT = 2,
+    FTGP_POLICY_SCALARS = 0, FTGP_POLICY_W1 = 4, FTGP_POLICY_B1 = 6148, FTGP_POLICY_W2 = 6212, FTGP_POLICY_B2 = 10308,
+    FTGP_POLICY_W3 = 10372, FTGP_POLICY_B3 = 10500, FTGP_POLICY_FLOATS = 10504
+};
+typedef struct {
+    const float* weights;        /* device float[npolicies][FTGP_POLICY_FLOATS] */
+    const int32_t* policy_id;    /* device int32[ncars] or NULL (every car on policy 0) */
+    int32_t npolicies;           /* >= 1 */
+    int32_t reserved;
+} ftgp_policy_args;
+/* ftgp_drivers_params plus the policy bank: policy NULL is exactly ftgp_drivers_params; with a bank, qpos (device
+ * double[ncars][FTGP_NQ]) and qvel (double[ncars][FTGP_NV]) give the inputs x[90..92].  The weights and ids are read by
+ * every call (and every graph-replayed tick of ftgp_tick_policy), so a bank rewritten in place in stream order takes
+ * effect on the next one.  default_kind in 0..3; FTGP_DRIVER_POLICY needs a bank. */
+int ftgp_drivers_policy(const float* ranges, const int32_t* kind, int default_kind, const double* params,
+                        const ftgp_policy_args* policy, const double* qpos, const double* qvel, const int32_t* lap,
+                        double* ctrl, int64_t ncars, void* stream);
 
 /* ------------------------------------------------------------------ lap logic */
 /* Replaces custom.py:1340-1372.  lap: device int32[ncars][FTGP_LAP_FIELDS] (see enum),
@@ -262,6 +306,11 @@ int ftgp_tick_reload(const ftgp_tick_args* a, const ftgp_reload_args* r, int nti
  * included, so rewriting them in place, in stream order, takes effect on the next tick. */
 int ftgp_tick_params(const ftgp_tick_args* a, const ftgp_reload_args* r, const double* driver_params, int nticks,
                      void* stream);
+/* ftgp_tick_params whose POLICY cars run the bank (see ftgp_drivers_policy); ftgp_tick_params is this call with
+ * policy NULL, and launches exactly the kernels it launched before policies existed.  The cached graph is keyed on the
+ * bank's pointers and npolicies; the weights and ids are read by every tick. */
+int ftgp_tick_policy(const ftgp_tick_args* a, const ftgp_reload_args* r, const double* driver_params,
+                     const ftgp_policy_args* policy, int nticks, void* stream);
 /* enable != 0 (default): small fleets replay the captured tick; 0: every tick is issued launch by launch.
  * Returns the previous setting (for A/B timing in the bench). */
 int ftgp_tick_use_graphs(int enable);
