@@ -14,10 +14,11 @@
 // kinematics / CRB / RNE of the wheel and softener bodies) runs 4-wide with no communication; the root block is
 // reduced across the quad with two xor-shuffles per value and then handled redundantly by the four lanes, which
 // keeps every loop bound and branch quad-uniform (sums are bit-identical in the four lanes).
-// A warp holds 8 cars; per-lane state is ~1/4 of a car and ALL of the solver's persistent state is in shared
-// memory: lane-private slots in [slot][thread] layout (conflict-free), root parts of the dof vectors and the root
-// block of M once per car in [slot][car] layout (the four lanes read them as a broadcast).  1 250 B per lane, so
-// 160 lanes (40 cars) are resident per SM; the factorisation itself runs entirely in registers.
+// A warp holds 8 cars; per-lane state is ~1/4 of a car and ALL of the solver's persistent state is on chip: lane-private
+// slots in shared memory in [slot][thread] layout (conflict-free), root parts of the dof vectors and the root block of M
+// once per car in [slot][car] layout (the four lanes read them as a broadcast), the lane's border of M in tensor memory
+// (Q::mb_load_row / mb_store_row).  784 B of shared memory and 288 B of tensor memory per lane, so 256 lanes (64 cars)
+// are resident per SM; the factorisation itself runs entirely in registers.
 // Control flow is WARP-UNIFORM (and CTA-uniform at the Newton loop head): every lane of a warp reaches every
 // collective in the same order, so the quad reductions are plain full-mask shuffles and the warps of a CTA walk the
 // same code at the same time (one instruction-cache fill serves all of them).  A quad whose car has converged keeps
@@ -48,14 +49,19 @@ namespace mushr {
 
 // ---- shared-memory slots (doubles).  P: private to the lane, C: one copy per car --------------------------------
 constexpr int QP_MW = 0;             // 21  chain block of M, lower triangle
-constexpr int QP_MB = 21;            // 36  border of M: slot l x root dof j < 6 (column 6 of M's border is zero)
-constexpr int QP_CJ = 57;            // 18  wheel-ground contact Jacobian, row a x (3 root rotations, 3 chain slots)
-constexpr int QP_FRA = 75;           // 6   aref of the friction-loss rows of the chain slots
-constexpr int QP_EQ = 81;            // 3   Ackermann equality of a front chain: D (0: none), aref, dP/dx
-constexpr int QP_LIM = 84;           // 6   suspension / front steering limit: D[2] (0: inactive), aref[2], sign[2]
-constexpr int QP_WC = 90;            // 5   wheel-ground contact: D (0: none), aref[4]
-constexpr int QP_VEC = 95;           // 4 x 6 chain parts of the dof vectors below
+constexpr int QP_CJ = 21;            // 18  wheel-ground contact Jacobian, row a x (3 root rotations, 3 chain slots)
+constexpr int QP_FRA = 39;           // 6   aref of the friction-loss rows of the chain slots
+constexpr int QP_EQ = 45;            // 3   Ackermann equality of a front chain: D (0: none), aref, dP/dx
+constexpr int QP_LIM = 48;           // 6   suspension / front steering limit: D[2] (0: inactive), aref[2], sign[2]
+constexpr int QP_WC = 54;            // 5   wheel-ground contact: D (0: none), aref[4]
+constexpr int QP_VEC = 59;           // 4 x 6 chain parts of the dof vectors below
+constexpr int QP_SM_N = 83;          // the slots above are the ones the device keeps in shared memory
+constexpr int QP_MB = 83;            // 36  border of M: slot l x root dof j < 6 (column 6 of M's border is zero)
 constexpr int QP_N = 119;
+// The border of M is written once per step and read a row of six at a time, always through mb_load_row / mb_store_row
+// below.  A policy that has those members keeps it elsewhere (QuadDev: in tensor memory, which no kernel of the tick uses
+// otherwise; it frees 288 B of shared memory per lane) and there they are warp collectives; for a policy without them
+// (the host harnesses) the border is the private slots QP_MB ... QP_N - 1.
 constexpr int QC_MR = 0;             // 28  root block of M, lower triangle
 constexpr int QC_R6 = 28;            // 4   rows of root dof 6 (steering wheel): friction aref, limit D, aref, sign
 constexpr int QC_VEC = 32;           // 4 x 7 root parts of the dof vectors
@@ -89,10 +95,38 @@ template <int PS_, int CS_, bool CTA_LOCKSTEP>
 struct QuadDev {                     // po / co / ko: offsets (in doubles) of the lane's, the car's and the table's first slot
     static constexpr int PS = PS_, CS = CS_;
     int po, co, ko, w, qs;           // qs: position of the quad in the warp (lane & 28)
+    uint32_t tm;                     // tensor-memory address of the warp's border rows (tmem_border_addr)
     __device__ __forceinline__ double& P(int i) const { return quad_sm[po + i * PS]; }
     __device__ __forceinline__ double& C(int i) const { return quad_sm[co + i * CS]; }
     __device__ __forceinline__ double K(int i) const { return quad_sm[ko + i]; }
     __device__ __forceinline__ int lane() const { return w; }
+    // row l of the lane's border of M: 12 columns (six doubles as lo/hi words) from column 12 l of the thread's TMEM lane.
+    // tcgen05.ld / st are .sync.aligned warp collectives; the __syncwarp makes sure the warp arrives converged.  The wait
+    // sits in the same asm statement so that no use of the loaded registers can be scheduled before it.
+    __device__ __forceinline__ void mb_load_row(int l, double* b) const {
+        uint32_t r[12];
+        __syncwarp();
+        asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%12];\n\t"
+                     "tcgen05.ld.sync.aligned.32x32b.x4.b32 {%8, %9, %10, %11}, [%13];\n\t"
+                     "tcgen05.wait::ld.sync.aligned;"
+                     : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
+                       "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11])
+                     : "r"(tm + 12u * l), "r"(tm + 12u * l + 8u));
+#pragma unroll
+        for (int j = 0; j < 6; j++) b[j] = __hiloint2double((int)r[2 * j + 1], (int)r[2 * j]);
+    }
+    __device__ __forceinline__ void mb_store_row(int l, const double* b) const {
+        uint32_t r[12];
+#pragma unroll
+        for (int j = 0; j < 6; j++) { r[2 * j] = (uint32_t)__double2loint(b[j]); r[2 * j + 1] = (uint32_t)__double2hiint(b[j]); }
+        __syncwarp();
+        asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%2, %3, %4, %5, %6, %7, %8, %9};\n\t"
+                     "tcgen05.st.sync.aligned.32x32b.x4.b32 [%1], {%10, %11, %12, %13};\n\t"
+                     "tcgen05.wait::st.sync.aligned;"
+                     :: "r"(tm + 12u * l), "r"(tm + 12u * l + 8u), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]),
+                        "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11])
+                     : "memory");
+    }
     // collectives: called by all 32 lanes of the warp together (cany: by the whole CTA)
     __device__ __forceinline__ double sum(double v) const {
         v += __shfl_xor_sync(0xffffffffu, v, 1);
@@ -106,6 +140,19 @@ struct QuadDev {                     // po / co / ko: offsets (in doubles) of th
     __device__ __forceinline__ void sync() const { __syncwarp(); }
 };
 #endif
+
+template <class Q, class = void> struct HasMbRows { static constexpr bool value = false; };
+template <class Q> struct HasMbRows<Q, decltype(static_cast<const Q*>(nullptr)->mb_load_row(0, static_cast<double*>(nullptr)))> {
+    static constexpr bool value = true;
+};
+template <class Q> FT_HD void mb_load_row(const Q& qd, int l, double* b) {
+    if constexpr (HasMbRows<Q>::value) qd.mb_load_row(l, b);
+    else for (int j = 0; j < 6; j++) b[j] = qd.P(QP_MB + 6 * l + j);
+}
+template <class Q> FT_HD void mb_store_row(const Q& qd, int l, const double* b) {
+    if constexpr (HasMbRows<Q>::value) qd.mb_store_row(l, b);
+    else for (int j = 0; j < 6; j++) qd.P(QP_MB + 6 * l + j) = b[j];
+}
 
 FT_HDN void quad_const_entry(const ModelConsts& mc, int g, double* t) {      // g: 0..23 chain slot (w, l), 24: root dof 6
     const int p = g < 24 ? NR + g : 6;
@@ -378,7 +425,7 @@ FT_QN double rows_eval(const Q& qd, const QChassis& ch, int nch, int ww, QVec X,
     return cost;
 }
 
-// y = M X with M in shared memory, result in registers (root part replicated)
+// y = M X with M on chip (shared and tensor memory), result in registers (root part replicated)
 template <class Q>
 FT_QN void quad_mul(const Q& qd, QVec X, double* yr, double* yc) {
     double xr[NR], xc[NC], part[6];
@@ -390,8 +437,10 @@ FT_QN void quad_mul(const Q& qd, QVec X, double* yr, double* yc) {
         double s = 0;
 #pragma unroll
         for (int k = 0; k < NC; k++) s += qd.P(QP_MW + (l >= k ? tri(l, k) : tri(k, l))) * xc[k];
+        double b[6];
+        mb_load_row(qd, l, b);
 #pragma unroll
-        for (int j = 0; j < 6; j++) { const double b = qd.P(QP_MB + 6 * l + j); s += b * xr[j]; part[j] += b * xc[l]; }
+        for (int j = 0; j < 6; j++) { s += b[j] * xr[j]; part[j] += b[j] * xc[l]; }
         yc[l] = s;
     }
 #pragma unroll
@@ -443,8 +492,7 @@ FT_QN void quad_factor_solve(const Q& qd, const QChassis& ch, const QState& st, 
     for (int i = 0; i < 21; i++) W[i] = qd.P(QP_MW + i);
 #pragma unroll
     for (int l = 0; l < NC; l++) {
-#pragma unroll
-        for (int j = 0; j < 6; j++) B[l][j] = qd.P(QP_MB + 6 * l + j);
+        mb_load_row(qd, l, B[l]);
         B[l][6] = 0;
     }
 #pragma unroll
@@ -581,15 +629,16 @@ FT_QN void quad_factor_solve(const Q& qd, const QChassis& ch, const QState& st, 
 #pragma unroll
         for (int i = 0; i < k; i++) xr[i] -= R[tri(k, i)] * xr[k];
     }
-    // chain: x_c = W^-1 (b_c - B x_r) with the ORIGINAL border B, rebuilt from shared memory (keeping Y = L^-1 B
+    // chain: x_c = W^-1 (b_c - B x_r) with the ORIGINAL border B, read again from where it is stored (keeping Y = L^-1 B
     // alive across the root factorisation costs 84 registers and spills; rebuilding B x_r costs ~90 DFMA)
     {
         double t[NC];
 #pragma unroll
         for (int l = 0; l < NC; l++) {
-            double sacc = qd.P(V.p + l);
+            double sacc = qd.P(V.p + l), b[6];
+            mb_load_row(qd, l, b);
 #pragma unroll
-            for (int j = 0; j < 6; j++) sacc -= qd.P(QP_MB + 6 * l + j) * xr[j];
+            for (int j = 0; j < 6; j++) sacc -= b[j] * xr[j];
             t[l] = sacc;
         }
         t[1] -= eqb * xr[6];
@@ -908,7 +957,7 @@ FT_QN void quad_prepare(const Q& qd, const ModelConsts& mc, const double* qr, co
     { const double ay[3] = {Rsteer[1], Rsteer[4], Rsteer[7]}; for (int a = 0; a < 3; a++) cd[2][a] = ay[a]; cross3(cd[2] + 3, ay, off); }
 #pragma unroll
     for (int cc = 0; cc < 3; cc++) { const double ax[3] = {Rs[cc], Rs[3 + cc], Rs[6 + cc]}; for (int a = 0; a < 3; a++) cd[3 + cc][a] = ax[a]; cross3(cd[3 + cc] + 3, ax, off); }
-    // ---- composite-rigid-body mass matrix -> shared memory
+    // ---- composite-rigid-body mass matrix -> shared memory, its border -> Q::mb_store_row
     {
         double crbw[10], crb1[10], buf[6];
 #pragma unroll
@@ -931,8 +980,10 @@ FT_QN void quad_prepare(const Q& qd, const ModelConsts& mc, const double* qr, co
                 if (kk == l) s = (l == 1 && !fr) ? 1.0 : s + dof_armature(NR + l);      // rear dummy steering slot: unit diagonal
                 qd.P(QP_MW + tri(l, kk)) = s;
             }
+            double b[6];
 #pragma unroll
-            for (int j = 0; j < 6; j++) qd.P(QP_MB + 6 * l + j) = dot6q(cdr[j], buf);
+            for (int j = 0; j < 6; j++) b[j] = dot6q(cdr[j], buf);
+            mb_store_row(qd, l, b);
         }
     }
     // ---- bias forces (recursive Newton-Euler), smooth force
@@ -1221,12 +1272,12 @@ FT_HD void quad_store_chain(int w, double* dst, const double* c, int base) {   /
 }
 
 // ---- staged solve: a car that has not converged after `max_rounds` Newton rounds of its CTA is SUSPENDED (its solver
-// state -- exactly the shared-memory slots plus a few scalars -- goes to a record in global memory) and a later launch
-// packs the suspended cars of the whole fleet into fresh CTAs and goes on.  A CTA runs its cars in lock-step, so
-// without this every car pays for the slowest of its 54 neighbours: measured mean 2.1 Newton iterations per car,
+// state -- exactly the shared-memory slots and the border of M plus a few scalars -- goes to a record in global memory) and
+// a later launch packs the suspended cars of the whole fleet into fresh CTAs and goes on.  A CTA runs its cars in lock-step,
+// so without this every car pays for the slowest of its neighbours: measured mean 2.1 Newton iterations per car,
 // 4.5 per CTA (tools/iteration_stats.py).  The arithmetic a car sees does not change (results are bit-identical).
 constexpr int QREC_CH = QMAXCH * (1 + 4 + 18), QREC_W1 = 1 + 4 + 36, QREC_WW = 2 * QREC_W1;
-constexpr int QREC_LANE = QP_N + QREC_CH + QREC_WW + 2;    // per lane: private slots, body contacts, wheel-wall contact, (cost, gauss)
+constexpr int QREC_LANE = QP_N + QREC_CH + QREC_WW + 2;    // per lane: private slots (border of M included), body contacts, wheel-wall contact, (cost, gauss)
 constexpr int QREC_DOUBLES = 4 * QREC_LANE + QC_N + 10;    // + per-car slots + (c0, mask[4], nch[4], ww[4], info) packed below
 struct QStage {
     int max_rounds;              // Newton rounds this launch may spend (<= 0: unlimited)
@@ -1237,7 +1288,7 @@ struct QStage {
 template <class Q>
 FT_HD void quad_suspend(const Q& qd, const QChassis& ch, const QState& st, const StepInfo& info, double* rec) {
     const int w = qd.lane();
-    for (int i = 0; i < QP_N; i++) rec[4 * i + w] = qd.P(i);
+    for (int i = 0; i < QP_SM_N; i++) rec[4 * i + w] = qd.P(i);      // (the border: quad_suspend_border)
     double* r2 = rec + 4 * QP_N;
     {
         int k = 0;
@@ -1270,7 +1321,7 @@ FT_HD void quad_suspend(const Q& qd, const QChassis& ch, const QState& st, const
 template <class Q>
 FT_HD void quad_resume(const Q& qd, QChassis& ch, QState& st, StepInfo& info, const double* rec) {
     const int w = qd.lane();
-    for (int i = 0; i < QP_N; i++) qd.P(i) = rec[4 * i + w];
+    for (int i = 0; i < QP_SM_N; i++) qd.P(i) = rec[4 * i + w];      // (the border: quad_resume_border)
     const double* r3 = rec + 4 * QREC_LANE;
     for (int i = 0; i < QC_N; i++) qd.C(i) = r3[i];          // every lane writes the same values
     const double* r4 = r3 + QC_N;
@@ -1299,6 +1350,29 @@ FT_HD void quad_resume(const Q& qd, QChassis& ch, QState& st, StepInfo& info, co
     }
 }
 
+// The border of M travels with the record as well.  Its accessors are warp collectives, so these two are called by every
+// lane of the warp; on: this lane's car is the one suspended / resumed.
+template <class Q>
+FT_HD void quad_suspend_border(const Q& qd, double* rec, bool on) {
+    double* rb = rec + 4 * QP_MB + qd.lane();
+#pragma unroll
+    for (int l = 0; l < NC; l++) {
+        double b[6];
+        mb_load_row(qd, l, b);
+        if (on) for (int j = 0; j < 6; j++) rb[4 * (6 * l + j)] = b[j];
+    }
+}
+template <class Q>
+FT_HD void quad_resume_border(const Q& qd, const double* rec, bool on) {
+    const double* rb = rec + 4 * QP_MB + qd.lane();
+#pragma unroll
+    for (int l = 0; l < NC; l++) {
+        double b[6];
+        for (int j = 0; j < 6; j++) b[j] = on ? rb[4 * (6 * l + j)] : 0.0;
+        mb_store_row(qd, l, b);
+    }
+}
+
 // ---- the step -----------------------------------------------------------------------------------------------------
 // live = false: a padding quad (it re-does the last car so that it can take part in the collectives, and stores
 // nothing to global memory)
@@ -1317,6 +1391,7 @@ FT_STEP bool step_car_quad(const Q& qd, const ModelConsts& mc, double* qpos, dou
     qd.sync();                                                             // previous step's root state is in memory
     if (stage.resume) {
         if (live) quad_resume(qd, ch, st, info, stage.rec);
+        quad_resume_border(qd, stage.rec, live);
         qd.sync();
     } else {
         double qr[8], qc[7], vr[NR], vc[NC];
@@ -1424,6 +1499,7 @@ FT_STEP bool step_car_quad(const Q& qd, const ModelConsts& mc, double* qpos, dou
     }
     const bool suspended = mode == 4;                                      // the record takes the solver state
     qd.sync();
+    if (stage.rec) quad_suspend_border(qd, stage.rec, suspended && live);
     if (suspended && live) quad_suspend(qd, ch, st, info, stage.rec);
     // (a suspended quad still walks through the collectives below with the rest of its warp, then leaves)
     double xr[NR], xc[NC], ar[NR], ac[NC];

@@ -54,14 +54,27 @@ __device__ __forceinline__ int status_word(const StepInfo& info, int prev) {
 }
 
 // Quad-per-car: four lanes (one per wheel chain) advance one car, 8 cars per warp; see mushr_step_quad.cuh.
-// Shared memory: [slot][thread] for the lane-private slots, [slot][car] for the per-car slots, then the table of
-// friction-loss row constants.  1 072 B per lane: one 216-thread CTA (54 cars) per SM.
-template <int NT> constexpr size_t quad_smem_bytes() { return (size_t)(NT * QP_N + NT / 4 * QC_N + QK_N + 1) * sizeof(double); }
+// Shared memory: [slot][thread] for the lane-private slots below QP_SM_N, [slot][car] for the per-car slots, then the table of
+// friction-loss row constants: 784 B per lane.  The border of M (288 B per lane) is in tensor memory.  One 256-thread
+// CTA (64 cars, 201,312 B of shared memory, 255 registers per thread) per SM.
+template <int NT> constexpr size_t quad_smem_bytes() { return (size_t)(NT * QP_SM_N + NT / 4 * QC_N + QK_N + 1) * sizeof(double); }
+
+// Tensor memory: the CTA allocates 256 columns (of 512) and thread t keeps its border of M in TMEM lane t % 128, 72 columns
+// from column 128 (t / 128).  A warp may only touch the 32 lanes of its quarter (warp % 4), so warps w and w + 4 share
+// lanes and take different column halves.  No kernel of the package issues an MMA or uses TMEM otherwise, and shared
+// memory and registers admit one CTA per SM, so the allocation never waits.  A CTA that exits without freeing its columns
+// would stall the next one on that SM forever: the kernel below has no early exit, and frees them at its single end.
+constexpr int TMEM_COLS = 256;
+static_assert(12 * NC <= TMEM_COLS / 2, "a thread's border rows must fit its half of the allocation");
+__device__ __forceinline__ uint32_t tmem_border_addr(uint32_t base, int tid) {
+    const int warp = tid >> 5;
+    return base + ((uint32_t)(32 * (warp & 3)) << 16) + (uint32_t)(TMEM_COLS / 2) * (uint32_t)(warp >> 2);
+}
 
 // ONE kernel serves both launches of the staged solve, with ONE inlined copy of the step:
-//   resume = 0  the first launch: CTA b steps cars [54 b, 54 b + 54) of the (regrouped) fleet; a car that is not done after
+//   resume = 0  the first launch: CTA b steps cars [64 b, 64 b + 64) of the (regrouped) fleet; a car that is not done after
 //               max_rounds Newton rounds of its CTA is parked in its record (recs != NULL) and listed in list_out;
-//   resume = 1  the continuation: a persistent grid (one CTA per SM) packs the cars listed in list_in, 54 at a time,
+//   resume = 1  the continuation: a persistent grid (one CTA per SM) packs the cars listed in list_in, 64 at a time,
 //               restores their solver state from the records and goes on (max_rounds <= 0: to convergence).
 // Both paths run the same machine code for the solver, so a suspended and resumed car gets bit-identical results to one that
 // converges in a single launch: with two kernels (two inlined copies) the compiler contracted a few multiply-adds
@@ -75,12 +88,22 @@ step_quad_kernel(const uint32_t* __restrict__ blob, double* __restrict__ qpos, d
                  int32_t* __restrict__ status, double* __restrict__ recs, const int32_t* __restrict__ list_in,
                  const int32_t* __restrict__ count_in, int32_t* __restrict__ list_out, int32_t* __restrict__ count_out,
                  int max_rounds, int options, const uint8_t* __restrict__ world_flag, int cpw, int resume) {
+    static_assert(NT % 32 == 0 && NT <= 256, "TMEM accesses are warp collectives: whole warps, two per lane quarter");
+    static_assert(HasMbRows<QuadDev<NT, NT / 4, LOCK>>::value, "shared memory holds the first QP_SM_N private slots only");
+    __shared__ uint32_t tmem_base;
     const int tid = threadIdx.x, cib = tid >> 2;
-    constexpr int KO = NT * QP_N + NT / 4 * QC_N, CARS = NT / 4;
+    constexpr int KO = NT * QP_SM_N + NT / 4 * QC_N, CARS = NT / 4;
+    if (tid < 32) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
+                     :: "r"((uint32_t)__cvta_generic_to_shared(&tmem_base)), "n"(TMEM_COLS) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
     for (int g = tid; g < 25; g += NT) quad_const_entry(c_model, g, quad_sm + KO);
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     QuadDev<NT, NT / 4, LOCK> qd;
-    qd.w = tid & 3; qd.po = tid; qd.co = NT * QP_N + cib; qd.ko = KO; qd.qs = tid & 28;
+    qd.w = tid & 3; qd.po = tid; qd.co = NT * QP_SM_N + cib; qd.ko = KO; qd.qs = tid & 28; qd.tm = tmem_border_addr(tmem_base, tid);
     const int64_t nwork = resume ? (int64_t)*count_in : ncars;
     for (int64_t base = (int64_t)blockIdx.x * CARS; base < nwork; base += (int64_t)gridDim.x * CARS) {
         const int64_t e = base + cib;
@@ -107,6 +130,10 @@ step_quad_kernel(const uint32_t* __restrict__ blob, double* __restrict__ qpos, d
         if (!resume) break;                             // first launch: one batch per CTA
         __syncthreads();                                // the next batch reuses the shared-memory slots
     }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    if (tid < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem_base), "n"(TMEM_COLS) : "memory");
 }
 
 // The quad-per-car kernel runs the cars of a CTA in lock-step, so a CTA takes as many Newton rounds as its slowest
@@ -116,7 +143,7 @@ constexpr int NBIN = 16;
 // bit 10 of the status word: the car was within reach of a wall last step (the gate of quad_prepare).  Only such cars run the
 // wall probes, and a warp runs them if ANY of its 8 cars does -- so the cars near walls are kept together.
 __device__ __forceinline__ int order_bin(int st) { return min(st & 0xFF, 7) + ((st & 0x400) ? 8 : 0); }
-// (cars of a world flagged as coupled sit in the last bin whatever their status word says: inside the fused tick their solver
+// (cars of a world flagged as coupled sit in bin NBIN - 1 whatever their status word says: inside the fused tick their solver
 // is already running beside these kernels and rewrites those words)
 __device__ __forceinline__ int order_bin_of(const int32_t* __restrict__ status, const uint8_t* __restrict__ world_flag, int cpw, int64_t i) {
     if (world_flag && world_flag[i / cpw]) return NBIN - 1;
@@ -132,6 +159,11 @@ __global__ void order_hist_kernel(const int32_t* __restrict__ status, const uint
     __syncthreads();
     if (threadIdx.x < NBIN && h[threadIdx.x]) atomicAdd(&hist[threadIdx.x], h[threadIdx.x]);
 }
+// The bins are laid out in DESCENDING order: the CTAs of the slowest cars (near a wall, many Newton iterations) start in the
+// first wave, and the last, partly filled wave holds the quick ones (FTGP_AB_BIN_DESC=0: ascending, for tools/step_ab.py).
+#ifndef FTGP_AB_BIN_DESC
+#define FTGP_AB_BIN_DESC 1
+#endif
 __global__ void order_scatter_kernel(const int32_t* __restrict__ status, const uint8_t* __restrict__ world_flag, int cpw, int64_t ncars,
                                      const int32_t* __restrict__ hist, int32_t* __restrict__ cursor, int32_t* __restrict__ perm) {
     __shared__ int h[NBIN], base[NBIN];
@@ -143,7 +175,7 @@ __global__ void order_scatter_kernel(const int32_t* __restrict__ status, const u
     __syncthreads();
     if (threadIdx.x < NBIN) {
         int start = 0;
-        for (int b = 0; b < (int)threadIdx.x; b++) start += hist[b];
+        for (int b = 0; b < NBIN; b++) if (FTGP_AB_BIN_DESC ? b > (int)threadIdx.x : b < (int)threadIdx.x) start += hist[b];
         base[threadIdx.x] = start + (h[threadIdx.x] ? atomicAdd(&cursor[threadIdx.x], h[threadIdx.x]) : 0);
     }
     __syncthreads();
@@ -271,12 +303,10 @@ world_step_kernel(const uint32_t* __restrict__ blob, double* __restrict__ qpos, 
     }
 }
 
-// The production mapping is frozen: 216-thread CTAs (54 cars, 6 warps + 24 lanes), CTA-level lock-step of the Newton
+// The production mapping is frozen: 256-thread CTAs (64 cars, 8 full warps), CTA-level lock-step of the Newton
 // loop, cars regrouped by (last Newton iteration count, wall contact), staged solve with two Newton rounds in the first
 // launch (DESIGN.md 8 lists the measured alternatives; the A/B variants live in tests/host_harness, not in this library).
-// NOTE on the 24-lane tail warp: QuadDev's collectives use the full mask; lanes 24-31 of that warp do not exist (they
-// count as exited threads, which *_sync primitives ignore), and every quad is 4 lanes inside one warp.
-// (tools/build_variant.py compiles A/B variants of these three into separately named libraries for tools/step_ab.py;
+// (tools/build_variant.py compiles A/B variants of these into separately named libraries for tools/step_ab.py;
 // the shipped library always has the defaults)
 #ifndef FTGP_AB_LOCK
 #define FTGP_AB_LOCK true
@@ -284,7 +314,10 @@ world_step_kernel(const uint32_t* __restrict__ blob, double* __restrict__ qpos, 
 #ifndef FTGP_AB_ROUNDS
 #define FTGP_AB_ROUNDS 2
 #endif
-constexpr int STEP_NT = 216;
+#ifndef FTGP_AB_NT
+#define FTGP_AB_NT 256
+#endif
+constexpr int STEP_NT = FTGP_AB_NT;
 constexpr int STAGE_ROUNDS = FTGP_AB_ROUNDS;
 constexpr bool STEP_LOCK = FTGP_AB_LOCK;
 constexpr int64_t ORDER_MIN_CARS = 1024, STAGE_MIN_CARS = 4096;
@@ -395,7 +428,7 @@ int launch_step(const ftgp_geom* g, double* qpos, double* qvel, double* warm, co
     const int64_t nworlds = ncars / cpw;
     const bool fork_here = cpw > 1 && !o->world_inflight;          // (inside the fused tick the worlds are in flight already)
     if (fork_here && (rc = world_flag_launch(o, dev, qpos, lap, nworlds, cpw, stream))) return rc;
-    // cars grouped by (last Newton iteration count, wall contact) for the kernel that runs 54 cars in lock-step
+    // cars grouped by (last Newton iteration count, wall contact) for the kernel that runs 64 cars in lock-step
     const int32_t* perm = nullptr;
     if (reorder) {
         if (o->cap < ncars) {
