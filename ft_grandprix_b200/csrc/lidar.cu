@@ -329,6 +329,21 @@ enum { ST_IDLE = 0, ST_CHUNK = 1, ST_SWEEP = 2, ST_ADV = 3 };
 #ifndef FTGP_AB_REFILL
 #define FTGP_AB_REFILL 8            // idle lanes that trigger a refill
 #endif
+#ifndef FTGP_AB_LANESTATS
+#define FTGP_AB_LANESTATS 0         // 1: count rounds and active lanes per block into g_lane_stats (ftgp_lidar_lanestats)
+#endif
+#if FTGP_AB_LANESTATS
+// per block: rounds, lanes that entered; per inner loop: iterations, active lanes summed over them
+enum { LS_SETUP_ROUNDS, LS_SETUP_LANES, LS_WALK_ROUNDS, LS_WALK_LANES, LS_SWEEP_ROUNDS, LS_SWEEP_LANES, LS_HOP_ITERS,
+       LS_HOP_LANES, LS_LINE_ITERS, LS_LINE_LANES, LS_CELL_ITERS, LS_CELL_LANES, LS_N };
+__device__ unsigned long long g_lane_stats[LS_N];
+static int64_t g_lane_launch[4];      // shared memory, CTAs per SM, track staged, cars per batch of the last launch
+#define LANESTAT_ROUND(k, n) do { if (lane == 0) { ls[k]++; ls[(k) + 1] += (n); } } while (0)
+#define LANESTAT_LOOP(k) do { const unsigned am_ = __activemask(); if (lane == __ffs(am_) - 1) { ls[k]++; ls[(k) + 1] += __popc(am_); } } while (0)
+#else
+#define LANESTAT_ROUND(k, n) do { } while (0)
+#define LANESTAT_LOOP(k) do { } while (0)
+#endif
 constexpr int BATCH = 8;              // max cars per warp batch (a batch holds whole worlds of 1..8 cars)
 constexpr int MULTI_WORDS = BATCH * FTGP_NBEAMS + 64 + 66;   // per warp, multi-car worlds: nearest other-car hit per ray, beam window and running count per (car, other car)
 constexpr int FRAME_DOUBLES = 21;     // p[3], R[9], suspension travel [4], front steering angle [2], centre of the car's bounding sphere [3]
@@ -392,6 +407,9 @@ lidar_kernel(const uint32_t* __restrict__ blob, int lidar_words, const double* _
     const int64_t nbatch = (ncars + bsz - 1) / bsz;
     const double rx = -0.0525, rz = 0.065, lr = 0.030;   // mushr.em.xml:101-103
     const unsigned lt = (1u << lane) - 1u;
+#if FTGP_AB_LANESTATS
+    unsigned ls[LS_N] = {};
+#endif
 
     for (int64_t batch = (int64_t)blockIdx.x * warps_per_block + wib; batch < nbatch; batch += nwarps) {
         const int64_t base_car = batch * bsz;
@@ -496,6 +514,7 @@ lidar_kernel(const uint32_t* __restrict__ blob, int lidar_words, const double* _
             if (!refill && idle == 0xffffffffu) break;
             if (refill) {
                 const int r = next + __popc(idle & lt);
+                LANESTAT_ROUND(LS_SETUP_ROUNDS, min(__popc(idle), nrays - next));
                 next += __popc(idle);
                 if (L.state == ST_IDLE && r < nrays) {
                     // ---------------- ray set-up (fp64 pose math, then fp32 cell-relative coordinates)
@@ -589,6 +608,7 @@ lidar_kernel(const uint32_t* __restrict__ blob, int lidar_words, const double* _
                 else pick = (n_chunk >= FTGP_AB_HYST_B && n_chunk > 0) || n_sweep == 0 ? ST_CHUNK : ST_SWEEP;
                 mode = pick;
             }
+            if (pick == ST_CHUNK) LANESTAT_ROUND(LS_WALK_ROUNDS, n_chunk); else LANESTAT_ROUND(LS_SWEEP_ROUNDS, n_sweep);
             // ---------------- leave the previous chunk (exit side face, step of the chunk DDA) ...
             if (pick == ST_CHUNK && L.state == ST_ADV) {
                 bool done = false;
@@ -618,6 +638,7 @@ lidar_kernel(const uint32_t* __restrict__ blob, int lidar_words, const double* _
                 bool more = false;
                 const int entered = FTGP_AB_WALK_VOTE > 0 ? __popc(__activemask()) : 0;
                 for (int hop = 0;; hop++) {
+                    LANESTAT_LOOP(LS_HOP_ITERS);
                     if (FTGP_AB_WALK_MAX > 0 && hop == FTGP_AB_WALK_MAX) { more = true; break; }
                     if (FTGP_AB_WALK_VOTE > 0 && hop > 0 && __popc(__activemask()) * 4 < entered * FTGP_AB_WALK_VOTE) { more = true; break; }
                     const float tmx = L.inv_dgx != 0.f ? ((float)(L.ix - L.ix0 + (L.stepx > 0 ? 1 : 0)) - L.fx0) * L.inv_dgx : BIG;
@@ -700,6 +721,7 @@ lidar_kernel(const uint32_t* __restrict__ blob, int lidar_words, const double* _
                 const uint32_t* mk = L.major_x ? L.m + 15 : L.m;        // row-major masks for rows, transposed for columns
                 const int nline = L.major_x ? L.nrow : L.ncol;          // vertices per line
                 for (int hop = 0;; hop++) {
+                    LANESTAT_LOOP(LS_LINE_ITERS);
                     float s0 = 0.f, s1 = L.span;
                     if (L.inv_dM != 0.f) {
                         const float e0 = ((float)(L.c + (L.sg > 0 ? 0 : 1)) - L.Ma) * L.inv_dM;
@@ -721,6 +743,7 @@ lidar_kernel(const uint32_t* __restrict__ blob, int lidar_words, const double* _
                 }
                 float found = BIG;
                 while (cand && found == BIG) {
+                    LANESTAT_LOOP(LS_CELL_ITERS);
                     const int k = L.dm >= 0.f ? __ffs(cand) - 1 : 31 - __clz(cand);
                     cand &= ~(1u << k);
                     const uint32_t a2 = (lineA >> k) & 3u, b2 = (lineB >> k) & 3u;
@@ -743,6 +766,10 @@ lidar_kernel(const uint32_t* __restrict__ blob, int lidar_words, const double* _
             }
         }
     }
+#if FTGP_AB_LANESTATS
+    for (int k = 0; k < LS_N; k++)
+        if (ls[k]) atomicAdd(&g_lane_stats[k], (unsigned long long)ls[k]);
+#endif
 }
 
 static int ensure_beams(int device) {
@@ -782,8 +809,20 @@ int launch_lidar(const ftgp_geom* g, const double* qpos, int64_t stride, const i
         FTGP_CUDA(cudaFuncSetAttribute(lidar_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     }
     int rc = ensure_beams(dev); if (rc) return rc;
-    int per_sm = (int)std::min<size_t>(4, (227 * 1024) / (smem + 1024));
-    if (per_sm < 1) per_sm = 1;
+    // CTAs that can be resident on one SM at once, registers included: at 512 threads the kernel's registers leave room
+    // for one.  The grid is one wave of those, and the batch size below fills it; counting the shared memory alone
+    // gave 2, i.e. a second wave of CTAs queued behind the first and half the cars per batch.
+    static size_t occ_smem[16][2];
+    static int occ_ctas[16][2];
+    const int multi = cpw > 1;
+    int per_sm = 1;
+    if (dev < 16 && occ_smem[dev][multi] == smem && occ_ctas[dev][multi] > 0) per_sm = occ_ctas[dev][multi];
+    else {
+        FTGP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, multi ? lidar_kernel<true> : lidar_kernel<false>,
+                                                                threads, smem));
+        per_sm = std::max(1, std::min(4, per_sm));
+        if (dev < 16) { occ_smem[dev][multi] = smem; occ_ctas[dev][multi] = per_sm; }
+    }
     int nsm = dev < 16 ? sm_count[dev] : 148;
     // cars per warp batch: 8 for big fleets (best lane utilisation), fewer when the fleet would not fill the GPU
     int wpb = BATCH / cpw;                                      // whole worlds per batch
@@ -800,6 +839,9 @@ int launch_lidar(const ftgp_geom* g, const double* qpos, int64_t stride, const i
                                                              ncars, cpw, bsz, stage, ranges, min_range);
     count_launch();
     FTGP_CUDA(cudaGetLastError());
+#if FTGP_AB_LANESTATS
+    g_lane_launch[0] = (int64_t)smem; g_lane_launch[1] = per_sm; g_lane_launch[2] = stage; g_lane_launch[3] = bsz;
+#endif
     return FTGP_OK;
 }
 
@@ -847,3 +889,16 @@ extern "C" int ftgp_lidar_host(const ftgp_geom* g, const double* qpos, int64_t q
     FTGP_CUDA(cudaStreamSynchronize(s));
     return FTGP_OK;
 }
+
+#if FTGP_AB_LANESTATS
+// A/B builds only (tools/lidar_ab.py): out[0..LS_N) = the counters summed since the last call, which zeroes them,
+// then shared memory, CTAs per SM, track staged, cars per batch of the last launch.
+extern "C" int ftgp_lidar_lanestats(unsigned long long* out) {
+    FTGP_CUDA(cudaDeviceSynchronize());
+    FTGP_CUDA(cudaMemcpyFromSymbol(out, g_lane_stats, sizeof g_lane_stats));
+    const unsigned long long zero[LS_N] = {};
+    FTGP_CUDA(cudaMemcpyToSymbol(g_lane_stats, zero, sizeof zero));
+    for (int k = 0; k < 4; k++) out[LS_N + k] = (unsigned long long)g_lane_launch[k];
+    return FTGP_OK;
+}
+#endif
